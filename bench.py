@@ -11,6 +11,10 @@ sharded by utterance, no data-path collective); rank 0 prints ONE JSON line.
   e2e       same metric through the host-facing API: pinned host buffers, H2D + D2H in the timed region
   roofline  dominant kernel (avse_forward4_kernel): algorithmic bytes / CUDA-event duration vs MEASURED_PEAKS.json
   cpu_baseline / --impl reference: the float64 CPU restatement of the reference path (oracle/), timed on host cores
+
+--dump-outputs DIR writes what the timed path returned in its last step (mixed / speech / noise log-mel slices, mixed PCM,
+and the inverse section's reconstructed PCM from those outputs) for a seeded sample of utterances.  The inputs depend only on the arguments,
+so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -27,6 +31,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark leaves the tree as it found it (it may be read-only)
 
 SR, FPS, SLICE_MS = 16000, 25.0, 200
 UTT_SECONDS = 3.0
@@ -58,7 +63,15 @@ def parse_args():
     ap.add_argument("--corpus", type=int, default=0,
                     help="BASELINE configs[2]: a corpus of this many utterances sharded contiguously by utterance over the ranks "
                          "(engine.shard_range, strong scaling); a step is one pass over the rank's whole shard in launches of --batch")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write rank 0's outputs of the last timed step (and their inverse) as DIR/<name>.npy, float32, "
+                         "for a fixed seeded sample of utterances of at most 64 MB in all")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -408,6 +421,27 @@ def corpus_batch(torch, n, device, base_seed):
     return speech, noise
 
 
+DUMP_BYTES = 64 * 10 ** 6
+DUMP_KEYS = ("mixed", "speech", "noise", "mixed_pcm")
+
+
+def dump_rows(n, bytes_per_row):
+    """--dump-outputs: a fixed, seeded sample of utterance indices in [0, n), ascending, whose outputs fit DUMP_BYTES."""
+    import numpy as np
+    k = max(1, min(n, DUMP_BYTES // bytes_per_row))
+    return np.sort(np.random.RandomState(0).choice(n, k, replace=False))
+
+
+def dump_outputs(directory, outs, launch, rows, keys=DUMP_KEYS):
+    """Write utterances `rows` of the per-launch output dicts `outs` (utterance i is row i % launch of outs[i // launch])
+    as directory/<key>.npy in float32."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for k in keys:
+        a = np.concatenate([outs[i // launch][k][i % launch:i % launch + 1].cpu().numpy() for i in rows])
+        np.save(os.path.join(directory, k + ".npy"), a.astype(np.float32))
+
+
 def run_corpus(args, torch, dist, eng, eng_mod, device, rank, world):
     """BASELINE configs[2]: N utterances sharded contiguously by utterance over the ranks (engine.shard_range), no collective on
     the data path.  One step = one pass over the rank's whole shard (resident in HBM), in launches of at most --batch utterances.
@@ -442,6 +476,10 @@ def run_corpus(args, torch, dist, eng, eng_mod, device, rank, world):
     e1.record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    rows = None
+    if args.dump_outputs and rank == 0:
+        rows = dump_rows(n, 4 * (3 * N_VIDEO_SLICES * 80 * 20 + L))
+        dump_outputs(args.dump_outputs, outs, launch, rows)
     t = torch.tensor([e0.elapsed_time(e1)], device=device, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -467,6 +505,8 @@ def run_corpus(args, torch, dist, eng, eng_mod, device, rank, world):
                      "note": "whole step of the largest shard (per-kernel figures: the default workload's line)"},
         "gpu_launches": 3 * len(outs) * args.steps, "clocks": clocks, "cpu_baseline": None, "e2e": None,
     }
+    if rows is not None:
+        line["dump_outputs"] = {"dir": args.dump_outputs, "rows": rows.tolist()}
     if rank == 0:
         print(json.dumps(line), flush=True)
     if world > 1:
@@ -554,6 +594,11 @@ def main():
     e1.record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    rows = None
+    if args.dump_outputs and rank == 0:
+        # row budget includes the reconstructed PCM of the inverse section (shorter than L)
+        rows = dump_rows(B, 4 * (3 * N_VIDEO_SLICES * 80 * 20 + 2 * L))
+        dump_outputs(args.dump_outputs, [out], B, rows)
     ms_total = e0.elapsed_time(e1)
     k_ms = sum(a.elapsed_time(b) for a, b in zip(ev_k0, ev_k1)) / args.steps
     tmax = torch.tensor([ms_total, k_ms], device=device, dtype=torch.float64)
@@ -589,6 +634,8 @@ def main():
         "data": "synthetic", "config": workload_config(B, world), "roofline": roofline,
         "gpu_launches": 3 * args.steps, "clocks": clocks, "host_cpus_bound_to_gpu_numa_node": numa,
     }
+    if rows is not None:
+        line["dump_outputs"] = {"dir": args.dump_outputs, "rows": rows.tolist()}
 
     # ---------------- steady state: the same step back to back for >= --sustain-s seconds ----------------
     if args.sustain_s > 0:
@@ -636,6 +683,10 @@ def main():
             eng.reconstruct(mixed_pcm, mel)
         i1.record()
         barrier()
+        if rows is not None:
+            # one more call on the same inputs, after the timed region: holding each timed call's output alive would change
+            # what the allocator does inside it
+            dump_outputs(args.dump_outputs, [{"recon": eng.reconstruct(mixed_pcm, mel)}], B, rows, keys=("recon",))
         inv_ms = i0.elapsed_time(i1) / args.steps
         tinv = torch.tensor([inv_ms], device=device, dtype=torch.float64)
         if world > 1:

@@ -1,9 +1,8 @@
 """Test scaffolding for the drop-in tests (tests/test_dropin_speech_enhancer.py): a synthetic GRID-like dataset tree on
-disk, stand-ins for the third-party / out-of-scope modules that /root/reference/speech_enhancer.py imports (mediaio.ffmpeg,
-mediaio.video_io, facedetection, network), and -- for the CPU-only run -- an engine double backed by the float64 oracle.
+disk, stand-ins for the third-party / out-of-scope modules that the mirror's video front end imports (mediaio.video_io,
+facedetection) and for the reference's Keras network, the reference's speech_enhancer.py call sequence restated, and --
+for the CPU-only run -- an engine double backed by the float64 oracle.
 TEST INFRASTRUCTURE: nothing here is imported by the product."""
-import importlib
-import importlib.util
 import os
 import pickle
 import sys
@@ -14,7 +13,6 @@ import numpy as np
 
 from oracle import avse_oracle as O
 
-REFERENCE_DIR = "/root/reference"
 SR, FPS = 16000, 25.0
 PKG = "audio-visual-speech-enhancement_b200"
 
@@ -96,26 +94,18 @@ class FakeNetwork(object):
         return out
 
 
-def install_stubs(dp_module):
-    """sys.modules entries for everything speech_enhancer.py (se:1-14) and the mirror's preprocess_video_sample import."""
+def install_stubs():
+    """sys.modules entries for the third-party modules the mirror's preprocess_video_sample imports (dp:7, dp:9)."""
     mediaio = types.ModuleType("mediaio")
-    ffmpeg = types.ModuleType("mediaio.ffmpeg")
-
-    def merge(video_path, audio_path, out_path):
-        open(out_path, "wb").close()
-    ffmpeg.merge = merge
     video_io = types.ModuleType("mediaio.video_io")
     video_io.VideoFileReader = _VideoFileReader
-    mediaio.ffmpeg, mediaio.video_io = ffmpeg, video_io
+    mediaio.video_io = video_io
     facedetection = types.ModuleType("facedetection")
     fd_mod = types.ModuleType("facedetection.face_detection")
     fd_mod.FaceDetector = _FaceDetector
     facedetection.face_detection = fd_mod
-    network = types.ModuleType("network")
-    network.SpeechEnhancementNetwork = FakeNetwork
-    mods = {"mediaio": mediaio, "mediaio.ffmpeg": ffmpeg, "mediaio.video_io": video_io, "facedetection": facedetection,
-            "facedetection.face_detection": fd_mod, "network": network, "data_processor": dp_module}
-    saved = {k: sys.modules.get(k) for k in list(mods) + ["dataset", "speech_enhancer"]}
+    mods = {"mediaio": mediaio, "mediaio.video_io": video_io, "facedetection": facedetection, "facedetection.face_detection": fd_mod}
+    saved = {k: sys.modules.get(k) for k in mods}
     sys.modules.update(mods)
     return saved
 
@@ -128,18 +118,8 @@ def restore_modules(saved):
             sys.modules[k] = v
 
 
-def load_reference_module(name):
-    """Import /root/reference/<name>.py UNMODIFIED (from where it lies; nothing is copied)."""
-    path = os.path.join(REFERENCE_DIR, name + ".py")
-    spec = importlib.util.spec_from_file_location(name, path)
-    mod = importlib.util.module_from_spec(spec)
-    sys.modules[name] = mod
-    spec.loader.exec_module(mod)
-    return mod
-
-
 # ---------------------------------------------------------------------------------------------
-# the call sequence of se:17-28 / se:61-88 restated for the GPU box, where /root/reference does not exist
+# the call sequence of se:17-28 / se:61-88, restated
 # ---------------------------------------------------------------------------------------------
 AudioVisualEntry = namedtuple("AudioVisualEntry", ["speaker_id", "audio_path", "video_path"])
 
@@ -179,8 +159,8 @@ class CallSequenceDriver(object):
 
 
 # ---------------------------------------------------------------------------------------------
-# CPU-only engine double (oracle-backed) so that the unmodified reference can be driven through the mirror where there
-# is no GPU.  It implements exactly the engine surface data_processor.py touches.
+# CPU-only engine double (oracle-backed) so that the call sequence can be driven through the mirror where there is no
+# GPU.  It implements exactly the engine surface data_processor.py touches.
 # ---------------------------------------------------------------------------------------------
 class OracleEngineDouble(object):
     import torch as _torch

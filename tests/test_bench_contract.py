@@ -6,6 +6,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -39,9 +40,21 @@ def test_reference_arm_other_ranks_stay_silent():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_argument_errors():
+    for args in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "x"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + args, capture_output=True, text=True, timeout=300, cwd=ROOT)
+        assert r.returncode == 2 and "error:" in r.stderr and r.stdout == ""
+
+
 @pytest.mark.gpu
-def test_gpu_arm_line_small_batch():
-    d = _run(["--batch", "16", "--steps", "3", "--warmup", "3", "--cpu-sample", "8"])
+def test_gpu_arm_line_small_batch(tmp_path):
+    d = _run(["--batch", "16", "--steps", "3", "--warmup", "3", "--cpu-sample", "8", "--dump-outputs", str(tmp_path)])
+    assert d["dump_outputs"]["rows"] == list(range(16))                # the whole small batch fits the 64 MB budget
+    shapes = {"mixed": (16, 15, 80, 20), "speech": (16, 15, 80, 20), "noise": (16, 15, 80, 20), "mixed_pcm": (16, 48000),
+              "recon": (16, 47840)}
+    for name, shape in shapes.items():
+        a = np.load(str(tmp_path / (name + ".npy")))
+        assert a.shape == shape and a.dtype == np.float32 and np.isfinite(a).all(), name
     assert BASE_KEYS <= set(d) and "impl" not in d
     assert d["n_gpus"] == 1 and d["steps"] == 3 and d["warmup"] >= 3 and d["scaling"] == "weak" and d["dtype"] == "f32" and d["data"] == "synthetic"
     rf = d["roofline"]

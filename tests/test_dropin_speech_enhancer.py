@@ -1,21 +1,19 @@
 """SURVEY 8 rows a9 / a10: the mirror module is a drop-in for `import data_processor` in the reference's own entry points.
 
-* `test_unmodified_reference_speech_enhancer_runs_on_the_mirror` (CPU, this container): loads /root/reference/speech_enhancer.py
-  and dataset.py UNMODIFIED from where they lie, with sys.modules["data_processor"] = the mirror and stand-ins for the
-  out-of-scope third-party imports (mediaio.ffmpeg / video_io, facedetection, the Keras network), and runs the reference's
-  own `preprocess(args)` (se:17-28) and `predict(args)` (se:61-88) on a synthetic dataset tree.  There is no GPU here and
-  the product has no CPU path, so the engine behind the mirror is an oracle-backed test double: what this test pins is the
-  module surface (names, positional signatures, return types, pickling, in-place mutation, skip-on-failure).
-* `test_dropin_call_sequence_on_gpu` (-m gpu, the B200 box, where /root/reference does not exist): the same call sequence
-  -- through the unmodified reference file when it is present, otherwise through tests.dropin_support.CallSequenceDriver,
-  which restates se:25-28 / se:66-83 call for call -- on the REAL CUDA path, checked against the float64 oracle.
+The reference's speech_enhancer.py `preprocess(args)` (se:17-28) and `predict(args)` (se:61-88) are restated call for call
+by tests.dropin_support.CallSequenceDriver (se:25-28 / se:66-83), with stand-ins for the out-of-scope third-party imports
+(mediaio.video_io, facedetection, the Keras network), and run on a synthetic dataset tree:
+
+* `test_speech_enhancer_call_sequence_runs_on_the_mirror` (CPU): the product has no CPU path, so the engine behind the
+  mirror is an oracle-backed test double: what this test pins is the module surface (names, positional signatures, return
+  types, pickling, in-place mutation).
+* `test_dropin_call_sequence_on_gpu` (-m gpu): the same call sequence on the REAL CUDA path, checked against the float64
+  oracle.
 """
-import argparse
-import glob
 import importlib
+import json
 import os
 import pickle
-import random
 
 import numpy as np
 import pytest
@@ -24,7 +22,7 @@ from oracle import avse_oracle as O
 from tests import dropin_support as D
 
 TOL_DB, TOL_PCM = 1e-3, 1e-4
-HAVE_REFERENCE = os.path.exists(os.path.join(D.REFERENCE_DIR, "speech_enhancer.py"))
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def _oracle_sample(sample):
@@ -65,53 +63,35 @@ def _check_enhanced_wav(path, sample_before_predict, predicted, tol_lsb):
     assert np.max(np.abs(got.astype(np.int32) - want.astype(np.int32))) <= tol_lsb
 
 
-def _args(paths, **kw):
-    base = dict(base_dir=paths["base"], data_name="d", dataset_dir=paths["data"], noise_dirs=[paths["noise"]], speakers=None,
-                ignored_speakers=None, model="m", gpus=1)
-    base.update(kw)
-    return argparse.Namespace(**base)
-
-
-def _run_reference_entry_points(dp, paths, tol_db, tol_pcm, tol_lsb):
-    """preprocess(args) then predict(args) of the UNMODIFIED /root/reference/speech_enhancer.py against module `dp`."""
-    saved = D.install_stubs(dp)
+def _run_call_sequence(dp, paths, tol_db, tol_pcm, tol_lsb, tol_video):
+    """preprocess then predict of the reference's speech_enhancer.py against module `dp`: int16 WAVs on disk -> pickled
+    Samples -> enhanced WAVs."""
+    saved = D.install_stubs()
     try:
-        D.load_reference_module("dataset")
-        se = D.load_reference_module("speech_enhancer")
-        assert se.data_processor is dp
-        random.seed(3)
-        se.preprocess(_args(paths))                                                     # se:17-28
-        assets = se.AssetManager(paths["base"])
-        samples = se.load_preprocessed_blob(assets.get_preprocessed_blob_path("d"))     # pickled list of mirror Samples
+        drv = D.CallSequenceDriver(dp)
+        blob = os.path.join(paths["base"], "d.pkl")
+        drv.preprocess(paths, blob)
+        with open(blob, "rb") as fd:
+            samples = pickle.load(fd)
         _check_samples(samples, tol_db, tol_pcm)
         # what `train` leaves behind for predict (se:45-56): the normaliser built with the reference constructor and pickled
-        assets.create_model("m")
-        video, mixed, speech = se.make_sample_set(samples)
-        normalizer = dp.VideoNormalizer(video)
-        with open(assets.get_normalization_cache_path("m"), "wb") as fd:
-            pickle.dump(normalizer, fd)
-        D.FakeNetwork.predictions.clear()
-        se.predict(_args(paths))                                                        # se:61-88
-        wavs = sorted(glob.glob(os.path.join(paths["base"], "out", "m", "d", "*", "s1", "*", "enhanced.wav")))
-        assert len(wavs) == len(samples)
-        by_dir = {os.path.basename(os.path.dirname(w)).split("_")[0]: w for w in wavs}
-        for s in samples:
-            clip = os.path.splitext(os.path.basename(s.video_file_path))[0]
-            predicted = (np.asarray(s.mixed_spectrograms, dtype=np.float32) * 0.9 - 3.0).astype(np.float32)   # FakeNetwork.predict
-            _check_enhanced_wav(by_dir[clip], s, predicted, tol_lsb)
-            assert os.path.exists(os.path.join(os.path.dirname(by_dir[clip]), "mixture.wav"))
-        # normalisation happened in place on the unpickled samples (se:73) with the reference's statistics
-        allv = np.concatenate([s.video_samples for s in samples], axis=0)
-        mean, std = np.mean(allv, axis=(0, 3)), np.std(allv, axis=(0, 3))
-        probe = samples[0].video_samples.copy()
-        normalizer.normalize(probe)
-        assert np.allclose(probe, (samples[0].video_samples - mean[None, :, :, None]) / std[None, :, :, None], atol=2e-5)
+        video = np.concatenate([s.video_samples for s in samples], axis=0)
+        norm_path = os.path.join(paths["base"], "normalization.pkl")
+        with open(norm_path, "wb") as fd:
+            pickle.dump(dp.VideoNormalizer(video), fd)
+        outs = drv.predict(blob, norm_path, paths["base"])
+        assert len(outs) == len(samples)
+        for sample, predicted, wav in outs:
+            _check_enhanced_wav(wav, sample, predicted, tol_lsb)
+        # VideoNormalizer == numpy statistics (dp:201-212); normalised in place by predict (se:73)
+        mean, std = np.mean(video, axis=(0, 3)), np.std(video, axis=(0, 3))
+        first = [s for s in samples if s.video_file_path == outs[0][0].video_file_path][0]
+        assert np.allclose(outs[0][0].video_samples, (first.video_samples - mean[None, :, :, None]) / std[None, :, :, None], atol=tol_video)
     finally:
         D.restore_modules(saved)
 
 
-@pytest.mark.skipif(not HAVE_REFERENCE, reason="/root/reference is not present on this box")
-def test_unmodified_reference_speech_enhancer_runs_on_the_mirror(tmp_path, monkeypatch):
+def test_speech_enhancer_call_sequence_runs_on_the_mirror(tmp_path, monkeypatch):
     dp = importlib.import_module(D.PKG + ".data_processor")
     eng_mod = importlib.import_module(D.PKG + ".engine")
     doubles = {}
@@ -125,10 +105,9 @@ def test_unmodified_reference_speech_enhancer_runs_on_the_mirror(tmp_path, monke
     monkeypatch.setattr(dp, "get_engine", get_engine)                      # no GPU here: oracle-backed engine double
     monkeypatch.setattr(eng_mod, "VideoNormalizer", D.NumpyVideoNormalizerDouble)
     paths = D.build_dataset(str(tmp_path))
-    _run_reference_entry_points(dp, paths, tol_db=1e-4, tol_pcm=1e-6, tol_lsb=1)
+    _run_call_sequence(dp, paths, tol_db=1e-4, tol_pcm=1e-6, tol_lsb=1, tol_video=2e-5)
 
 
-@pytest.mark.skipif(not HAVE_REFERENCE, reason="/root/reference is not present on this box")
 def test_reference_call_forms_bind(tmp_path, monkeypatch):
     """The exact call forms the reference uses (dp:135-137, dp:160-162, dp:189, se:25, se:45, se:81) bind against the mirror's
     signatures: same positional order, same defaults."""
@@ -149,9 +128,10 @@ def test_reference_call_forms_bind(tmp_path, monkeypatch):
     assert list(inspect.signature(dp.VideoNormalizer.__init__).parameters) == ["self", "video_samples"]   # se:45
     assert list(inspect.signature(dp.VideoNormalizer.normalize).parameters) == ["self", "video_samples"]  # se:46, se:73
     # the reference module's public names all exist on the mirror
-    src = open(os.path.join(D.REFERENCE_DIR, "data_processor.py")).read()
-    import re
-    for name in re.findall(r"^(?:def|class) (\w+)", src, flags=re.M) + ["Sample"]:
+    with open(os.path.join(GOLD, "reference_data_processor_names.json")) as fd:
+        names = json.load(fd)["names"]
+    assert len(names) == 11
+    for name in names:
         assert hasattr(dp, name), name
     assert dp.Sample._fields == ("speaker_id", "video_file_path", "speech_file_path", "noise_file_path", "video_samples",
                                  "mixed_spectrograms", "speech_spectrograms", "noise_spectrograms", "mixed_signal", "video_frame_rate")
@@ -162,31 +142,7 @@ def test_dropin_call_sequence_on_gpu(tmp_path):
     """The real CUDA path under the reference's entry points: int16 WAVs on disk -> pickled Samples -> enhanced WAVs."""
     dp = importlib.import_module(D.PKG + ".data_processor")
     paths = D.build_dataset(str(tmp_path))
-    if HAVE_REFERENCE:
-        _run_reference_entry_points(dp, paths, tol_db=TOL_DB, tol_pcm=TOL_PCM, tol_lsb=4)
-        return
-    saved = D.install_stubs(dp)
-    try:
-        drv = D.CallSequenceDriver(dp)
-        blob = os.path.join(paths["base"], "d.pkl")
-        drv.preprocess(paths, blob)
-        with open(blob, "rb") as fd:
-            samples = pickle.load(fd)
-        _check_samples(samples, TOL_DB, TOL_PCM)
-        video = np.concatenate([s.video_samples for s in samples], axis=0)
-        norm_path = os.path.join(paths["base"], "normalization.pkl")
-        with open(norm_path, "wb") as fd:
-            pickle.dump(dp.VideoNormalizer(video), fd)
-        outs = drv.predict(blob, norm_path, paths["base"])
-        assert len(outs) == len(samples)
-        for sample, predicted, wav in outs:
-            _check_enhanced_wav(wav, sample, predicted, tol_lsb=4)      # 1e-4 of int16 full scale = 3.3 LSB
-        # VideoNormalizer on the GPU == numpy statistics (dp:201-212); normalised in place by predict (se:73)
-        mean, std = np.mean(video, axis=(0, 3)), np.std(video, axis=(0, 3))
-        first = [s for s in samples if s.video_file_path == outs[0][0].video_file_path][0]
-        assert np.allclose(outs[0][0].video_samples, (first.video_samples - mean[None, :, :, None]) / std[None, :, :, None], atol=2e-4)
-    finally:
-        D.restore_modules(saved)
+    _run_call_sequence(dp, paths, TOL_DB, TOL_PCM, tol_lsb=4, tol_video=2e-4)      # 1e-4 of int16 full scale = 3.3 LSB
 
 
 @pytest.mark.gpu
