@@ -126,17 +126,26 @@ struct Inv8Warp {
 };
 }  // namespace
 
-extern "C" int emul_inverse8(const float* mel_slices, int n_slices, const float* pcm, int L, int valid, float* out, int out_cap,
-                             int chunks, int sample_rate, double fmin, double fmax) {
+// All three call forms of the I8 kernel, as avse_inverse sets them up:
+//   layout 0 (AVSE_LAYOUT_SLICES): mel [n_slices][80][20];  layout 1 (AVSE_LAYOUT_SPEC): mel [80][ld_t], n_frames of them used;
+//   phase == nullptr: the phase of the mixture pcm[L] (zeros from `valid` on);  otherwise the explicit phase [phase_frames][321]
+//   (complex64) of the EXT instantiation, and pcm / L / valid are unused.
+// The warp's shared memory persists across groups and chunks like the kernel's: nothing is re-zeroed between groups.
+extern "C" int emul_inverse8_ex(const float* mel, int layout, int n_slices, int n_frames, int ld_t, const float* pcm, int L, int valid,
+                                const float* phase, int phase_frames, float* out, int out_cap, int chunks, int sample_rate, double fmin,
+                                double fmax) {
     HostTables h;
     if (!build_tables(h, sample_rate, fmin, fmax)) return -2;
-    const int T = 1 + L / HOP;
-    const int T_use = n_slices * SPSS < T ? n_slices * SPSS : T;
+    if (layout != 0 && layout != 1) return -3;
+    const bool ext = phase != nullptr;
+    const int T = ext ? phase_frames : 1 + L / HOP;
+    const int t_mel = layout == 0 ? n_slices * SPSS : n_frames;
+    const int T_use = t_mel < T ? t_mel : T;
+    if (T_use < 2 || (layout == 1 && ld_t < T_use)) return -3;
     const int G = (T_use + I8_FPG - 1) / I8_FPG;
-    const int T_pad = I8_FPG * (G + 1);
     const int out_len = HOP * (T_use - 1);
     if (out_cap < out_len) return -1;
-    (void)T_pad;
+    const vec2* ph = reinterpret_cast<const vec2*>(phase);
 
     std::vector<vec2> tw(N1 * N2), twT(N1 * N2);
     for (int k1 = 0; k1 < N1; ++k1)
@@ -198,24 +207,33 @@ extern "C" int emul_inverse8(const float* mel_slices, int n_slices, const float*
             const int c_left = (T_use - tl.t0 + 1) >> 1;
             const int c_hi = skip_ffts ? (c_left < I8_NC ? c_left : I8_NC) : I8_NC;
             if (have) {
-                for (int lane = 0; lane < 32; ++lane) i8_coef_load(lane, mel_slices, 0, 0, tl.t0, T_use, w.cd[lane]);
-                const bool interior = i8_group_interior(tl);
-                const bool mirrored = AVSE_I8_REFLECT_FAST && !interior && i8_group_reflect_only(tl);
-                if (interior || mirrored) {
-                    for (int lane = 0; lane < 32; ++lane) {
-                        if (interior) { i8_load_raw(tl, lane, w.raw[lane]); i8_load_tail_raw(tl, lane, w.rt[lane]); }
-                        else { i8_load_raw_reflect(tl, lane, w.raw[lane]); i8_load_tail_raw_reflect(tl, lane, w.rt[lane]); }
+                for (int lane = 0; lane < 32; ++lane) i8_coef_load(lane, mel, layout, ld_t, tl.t0, T_use, w.cd[lane]);
+                if (!ext) {      // EXT: no pass 1 (and no pass 2 below), the explicit phase replaces the mixture's spectrum
+                    const bool interior = i8_group_interior(tl);
+                    const bool mirrored = AVSE_I8_REFLECT_FAST && !interior && i8_group_reflect_only(tl);
+                    if (interior || mirrored) {
+                        for (int lane = 0; lane < 32; ++lane) {
+                            if (interior) { i8_load_raw(tl, lane, w.raw[lane]); i8_load_tail_raw(tl, lane, w.rt[lane]); }
+                            else { i8_load_raw_reflect(tl, lane, w.raw[lane]); i8_load_tail_raw_reflect(tl, lane, w.rt[lane]); }
+                        }
+                        for (int lane = 0; lane < 32; ++lane) i8_pass1_main(lane, w.raw[lane], w.lc[lane], frames, c_lo, c_hi);
+                        for (int lane = 0; lane < 32; ++lane) i8_pass1_tail(lane, w.rt[lane], s_win, tw.data(), frames);
+                    } else {
+                        for (int lane = 0; lane < 32; ++lane) i8_pass1_edge(tl, lane, s_win, tw.data(), frames, c_lo, c_hi);
                     }
-                    for (int lane = 0; lane < 32; ++lane) i8_pass1_main(lane, w.raw[lane], w.lc[lane], frames, c_lo, c_hi);
-                    for (int lane = 0; lane < 32; ++lane) i8_pass1_tail(lane, w.rt[lane], s_win, tw.data(), frames);
-                } else {
-                    for (int lane = 0; lane < 32; ++lane) i8_pass1_edge(tl, lane, s_win, tw.data(), frames, c_lo, c_hi);
                 }
                 for (int lane = 0; lane < 32; ++lane) i8_coef_local(lane, h.spike.data(), w.cd[lane], xch);
                 for (int lane = 0; lane < 32; ++lane) i8_coef_finish(lane, h.spike.data(), w.cd[lane], xch, ybuf);
-                for (int it = 0; it < 4; ++it) {
+                if (ext)
+                    for (int lane = 0; lane < 32; ++lane) {
+                        const int tA = tl.t0 + 2 * (lane >> 3);
+                        const vec2* phA = tA < T_use ? ph + (size_t)tA * NBINS : nullptr;
+                        const vec2* phB = tA + 1 < T_use ? ph + (size_t)(tA + 1) * NBINS : nullptr;
+                        i8_stage_post<true>(lane, col.data(), ybuf, frames, phA, phB);
+                    }
+                for (int it = ext ? 2 : 0; it < 4; ++it) {
                     const int r = it & 1;
-                    if (it == 2)
+                    if (it == 2 && !ext)
                         for (int lane = 0; lane < 32; ++lane) i8_stage_post<false>(lane, col.data(), ybuf, frames, nullptr, nullptr);
                     if (2 * r + 1 < c_lo || 2 * r >= c_hi) continue;
                     for (int lane = 0; lane < 32; ++lane) {
@@ -246,6 +264,11 @@ extern "C" int emul_inverse8(const float* mel_slices, int n_slices, const float*
         }
     }
     return out_len;
+}
+
+extern "C" int emul_inverse8(const float* mel_slices, int n_slices, const float* pcm, int L, int valid, float* out, int out_cap,
+                             int chunks, int sample_rate, double fmin, double fmax) {
+    return emul_inverse8_ex(mel_slices, 0, n_slices, 0, 0, pcm, L, valid, nullptr, 0, out, out_cap, chunks, sample_rate, fmin, fmax);
 }
 
 // The I8 kernel's partitioned ("SPIKE") coefficient solve alone: dB slices [n_slices][80][20] -> c[t][80] for the 8 frames of group g.
