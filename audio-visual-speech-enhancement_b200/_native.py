@@ -44,12 +44,26 @@ class InverseArgs(_c.Structure):
     ]
 
 
+class PoolMixArgs(_c.Structure):
+    _fields_ = [
+        ("speech_pool", _c.c_void_p), ("speech_len", _c.c_void_p), ("speech_stride", _c.c_longlong), ("n_speech", _c.c_longlong),
+        ("noise_pool", _c.c_void_p), ("noise_len", _c.c_void_p), ("noise_stride", _c.c_longlong), ("n_noise", _c.c_longlong),
+        ("sample_format", _c.c_int),
+        ("speech_index", _c.c_void_p), ("noise_index", _c.c_void_p), ("noise_offset", _c.c_void_p), ("snr_db", _c.c_void_p),
+        ("B", _c.c_int), ("L", _c.c_int), ("n_slices", _c.c_int),
+        ("out_speech", _c.c_void_p), ("out_noise", _c.c_void_p), ("out_mixed", _c.c_void_p), ("out_stride", _c.c_longlong),
+        ("mixed_pcm", _c.c_void_p), ("pcm_stride", _c.c_longlong),
+        ("factor_out", _c.c_void_p), ("equalizer_out", _c.c_void_p),
+        ("max_key", _c.c_void_p), ("min_key", _c.c_void_p), ("bad_row_flag", _c.c_void_p),
+    ]
+
+
 EXPORTS = [
     "avse_create", "avse_destroy", "avse_last_error", "avse_version", "avse_get_filterbank",
     "avse_snr_factor", "avse_forward", "avse_floor_inplace", "avse_floor_gather", "avse_reset_max", "avse_max_db",
     "avse_inverse", "avse_inverse_work_elems", "avse_floor_inplace3", "avse_gather_rows",
     "avse_create_ex", "avse_get_geometry", "avse_inverse_work_elems_ctx",
-    "avse_video_stats", "avse_video_normalize", "avse_mse", "avse_magphase",
+    "avse_video_stats", "avse_video_normalize", "avse_mse", "avse_magphase", "avse_mix_pooled",
 ]
 
 
@@ -109,6 +123,8 @@ def load(build=True):
     lib.avse_magphase.restype = i32
     lib.avse_gather_rows.argtypes = [vp, vp, vp, vp, ll, ll, vp, ll, vp, vp, vp, vp, vp]
     lib.avse_gather_rows.restype = i32
+    lib.avse_mix_pooled.argtypes = [vp, _c.POINTER(PoolMixArgs), vp]
+    lib.avse_mix_pooled.restype = i32
     _lib = lib
     return lib
 

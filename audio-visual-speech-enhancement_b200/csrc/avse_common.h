@@ -85,6 +85,77 @@ AVSE_HD void warp_split_range(const WarpSplit& s, int block, int warp, int warps
 #endif
 }
 
+// ---------------------------------------------------------------------------------------------
+// Pooled pairs (avse_mix_pooled): row b of a batch mixes speech clip speech_index[b] with noise clip noise_index[b] read from
+// its sample noise_offset[b] on, n[i] = z[(off + i) mod Ln] for i < Ls -- dp:119-139 on (s, z rotated by off).  off = 0 is
+// the reference's own "double until long enough, then truncate" rule (dp:125-128).
+// ---------------------------------------------------------------------------------------------
+struct PoolRows {
+    const long long* speech_index;   // [B]; nullptr: identity rows (avse_forward / avse_snr_factor batches)
+    const long long* noise_index;    // [B]
+    const int* noise_offset;         // [B] or nullptr (0 for every row)
+    const int* speech_len;           // [n_speech] clip lengths (clamped to [0, speech_stride])
+    const int* noise_len;            // [n_noise]  clip lengths (clamped to [0, noise_stride])
+    long long speech_stride, noise_stride, n_speech, n_noise;
+    int* bad_row_flag;               // set to 1 by the statistics pass for every invalid row (caller zeroes it)
+};
+
+// One resolved row: element offsets of the two clips, their lengths and the noise phase.  An invalid row (an index out of
+// range, or off outside [0, Ln) -- which includes every empty noise clip) comes back as the empty pair: both lengths 0,
+// nothing is read, factor 0, every log-mel at the amin floor.
+struct PoolRow {
+    long long s_off, n_off;
+    int ls, ln, off;
+    bool ok;
+};
+
+AVSE_HD PoolRow pool_row(const PoolRows& p, int b) {
+    PoolRow r;
+    r.s_off = 0; r.n_off = 0; r.ls = 0; r.ln = 0; r.off = 0;
+    const long long si = p.speech_index[b], ni = p.noise_index[b];
+    r.ok = si >= 0 && si < p.n_speech && ni >= 0 && ni < p.n_noise;
+    if (!r.ok) return r;
+    long long ls = p.speech_len[si], ln = p.noise_len[ni];
+    ls = ls < 0 ? 0 : (ls < p.speech_stride ? ls : p.speech_stride);
+    ln = ln < 0 ? 0 : (ln < p.noise_stride ? ln : p.noise_stride);
+    const int off = p.noise_offset ? p.noise_offset[b] : 0;
+    r.ok = off >= 0 && off < ln;
+    if (!r.ok) return r;
+    r.s_off = si * p.speech_stride;
+    r.n_off = ni * p.noise_stride;
+    r.ls = (int)ls; r.ln = (int)ln; r.off = off;
+    return r;
+}
+
+// Sums of the noise n[i] = z[(off + i) mod Ln], i < n, of one pair (the SNR statistics, dp:130), in one of two regimes:
+//   Ln >= n: the window [off, off + n) of z, read directly as at most two contiguous ranges [off, off + len0) and [0, len1)
+//            (a 60 s noise under a 3 s speech reads 3 s of it, not 60);
+//   Ln <  n: one pass over the stored clip, sample j weighted q + (((j - off) mod Ln) < rem), n = q Ln + rem.
+struct NoiseSpan {
+    bool periodic;
+    int len0, len1;   // window regime
+    int q, rem;       // periodic regime
+};
+
+AVSE_HD NoiseSpan noise_span(int n, int Ln, int off) {
+    NoiseSpan w;
+    w.periodic = Ln < n;
+    if (w.periodic) {
+        w.q = n / Ln; w.rem = n - w.q * Ln; w.len0 = Ln; w.len1 = 0;
+    } else {
+        w.q = 0; w.rem = 0;
+        w.len0 = Ln - off < n ? Ln - off : n;
+        w.len1 = n - w.len0;
+    }
+    return w;
+}
+
+AVSE_HD int noise_weight(const NoiseSpan& w, int j, int Ln, int off) {    // periodic regime, 0 <= j, off < Ln
+    int d = j - off;
+    d += d < 0 ? Ln : 0;
+    return w.q + (d < w.rem ? 1 : 0);
+}
+
 #if defined(__CUDACC__)
 // Cooperative copy of a constant table (N4 16-byte words, 16-byte aligned) from global memory into registers at kernel start.
 // The persistent kernels fetch ALL their tables first and store them to shared memory afterwards: a rolled "load, store, next"

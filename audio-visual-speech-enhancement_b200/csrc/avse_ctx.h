@@ -33,7 +33,8 @@ struct avse_ctx {
     size_t gen_fwd_smem_set = 0, gen_inv_smem_set = 0;   // dynamic shared-memory opt-in already requested through this context
 };
 
-int avse_generic_forward(avse_ctx* ctx, const avse_forward_args* args, void* stream);
+// pool == nullptr: rows of args->speech / args->noise; otherwise avse_mix_pooled's row indirection into them (avse_common.h)
+int avse_generic_forward(avse_ctx* ctx, const avse_forward_args* args, const avse::PoolRows* pool, void* stream);
 int avse_generic_inverse(avse_ctx* ctx, const avse_inverse_args* args, void* stream);
 int avse_generic_frames(const avse::GenericGeo& q, int L);
 

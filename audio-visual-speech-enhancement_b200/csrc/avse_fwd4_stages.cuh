@@ -59,9 +59,9 @@ AVSE_HD void lane4_const_init(int lane, const float* s_win, const vec2* s_tw, La
 }
 
 // A group is "interior" when its four frames exist and need neither reflection nor zero padding, and -- for a
-// periodically tiled noise (dp:125-128, period_n > 0) -- when the group's 1 120 samples do not straddle a period
-// boundary.  nz_shift is then the offset that maps the group's sample indices into the stored period:
-// noise[i] = nz[i + nz_shift] for every i of the group.
+// periodically tiled noise (dp:125-128, period_n > 0, read from phase_n on) -- when the group's 1 120 samples do not
+// straddle a period boundary.  nz_shift is then the offset that maps the group's sample indices into the stored period:
+// noise[i] = nz[(phase_n + i) mod period_n] = nz[i + nz_shift] for every i of the group.
 // TILED = false compiles the period logic out (the common kernel instantiation: see avse_forward4_kernel).
 template <typename S, bool TILED>
 AVSE_HD bool group4_interior(const FwdTileT<S>& tl, int& nz_shift) {
@@ -69,9 +69,10 @@ AVSE_HD bool group4_interior(const FwdTileT<S>& tl, int& nz_shift) {
     const int a = tl.t0 * HOP - HALF;                       // first sample of the group
     if (!(tl.nz != nullptr && a >= 0 && (tl.t0 + 3) * HOP + HALF <= tl.vmin && tl.t0 + 3 < tl.T)) return false;
     if (TILED && tl.period_n > 0) {
-        const int q = a / tl.period_n;
-        if ((a + (F4 - 1) * HOP + NFFT - 1) / tl.period_n != q) return false;
-        nz_shift = -q * tl.period_n;
+        const int j = a + tl.phase_n;
+        const int q = j / tl.period_n;
+        if ((j + (F4 - 1) * HOP + NFFT - 1) / tl.period_n != q) return false;
+        nz_shift = tl.phase_n - q * tl.period_n;
     }
     return true;
 }
@@ -371,7 +372,7 @@ AVSE_HD void stage4_pass1_edge(const FwdTileT<S>& tl, int lane, const float* s_w
 #pragma unroll
         for (int j = 0; j < 16; ++j) {
             rs[j] = load_sample_edge(tl.sp, base + N2 * j, tl.L, tl.valid_s);
-            rn[j] = tl.gain * load_sample_edge(tl.nz, base + N2 * j, tl.L, tl.valid_n, TILED ? tl.period_n : 0);
+            rn[j] = tl.gain * load_sample_edge(tl.nz, base + N2 * j, tl.L, tl.valid_n, TILED ? tl.period_n : 0, TILED ? tl.phase_n : 0);
         }
         if (tl.mixed_pcm != nullptr && t_raw < tl.T) {
 #pragma unroll

@@ -102,25 +102,38 @@ struct FwdTileT {
     // after the unpack by STFT linearity.
     float gain;          // applied to the noise samples at load; 0 when nz == nullptr
     float factor;        // residual applied to the (gain-scaled) noise spectrum / mel sums; 0 when nz == nullptr
-    int period_n;        // dp:125-128: noise[i] = nz[i mod period_n] (the reference doubles the noise until it covers the
-                         // speech, then truncates: a periodic tiling); 0: nz covers [0, valid_n) itself
+    int period_n;        // dp:125-128: noise[i] = nz[(phase_n + i) mod period_n] (the reference doubles the noise until it covers
+                         // the speech, then truncates: a periodic tiling; phase_n != 0 only for pooled pairs, avse_mix_pooled);
+                         // 0: nz covers [0, valid_n) itself
+    int phase_n;         // 0 <= phase_n < period_n; 0 when period_n == 0
     float* mixed_pcm;    // [L] or nullptr: s + f*n (dp:133), zero-padded / truncated to L
 };
 using FwdTile = FwdTileT<float>;
 
+// The noise row of a pair, n[i] = nz[(phase + i) mod period] for i < valid_n: a window that does not wrap (phase + valid_n <=
+// period, or no period at all) is the contiguous row nz + phase, read with no modulo anywhere (period = phase = 0 on return).
+template <typename S>
+AVSE_HD void fit_noise_row(const S*& nz, int& period, int& phase, int valid_n) {
+    if (period <= 0 || phase + valid_n <= period) {
+        if (nz != nullptr) nz += phase;
+        period = 0;
+        phase = 0;
+    }
+}
+
 // Sample i of a periodically tiled noise (dp:125-128).  Out of line: the integer modulo is ~25 instructions and the edge
 // loaders are unrolled 16 x, which would put 400 cold instructions into the middle of the kernel's instruction stream.
 template <typename S>
-AVSE_HD_COLD float load_sample_periodic(const S* p, int i, int period) { return (float)p[i % period]; }
+AVSE_HD_COLD float load_sample_periodic(const S* p, int i, int period, int phase) { return (float)p[(i + phase) % period]; }
 
 template <typename S>
-AVSE_HD float load_sample_edge(const S* p, int i, int L, int valid, int period = 0) {
+AVSE_HD float load_sample_edge(const S* p, int i, int L, int valid, int period = 0, int phase = 0) {
     // np.pad(y, n_fft//2, mode='reflect') on the length-L (zero padded) signal
     i = i < 0 ? -i : i;
     i = i >= L ? 2 * (L - 1) - i : i;
     i = i < 0 ? 0 : i;
     if (p == nullptr || i >= valid) return 0.0f;
-    return period > 0 ? load_sample_periodic(p, i, period) : (float)p[i];
+    return period > 0 ? load_sample_periodic(p, i, period, phase) : (float)p[i];
 }
 
 // A group is "interior" when both of its frames exist and all their samples are present in both
@@ -188,7 +201,7 @@ AVSE_HD void stage_pass1_edge(const FwdTile& tl, int lane, const float* s_win2, 
 #pragma unroll
         for (int j = 0; j < 16; ++j)
             x[j] = cmake(load_sample_edge(tl.sp, base + N2 * j, tl.L, tl.valid_s),
-                         tl.gain * load_sample_edge(tl.nz, base + N2 * j, tl.L, tl.valid_n, tl.period_n));
+                         tl.gain * load_sample_edge(tl.nz, base + N2 * j, tl.L, tl.valid_n, tl.period_n, tl.phase_n));
         if (tl.mixed_pcm != nullptr && t_raw < tl.T) {
 #pragma unroll
             for (int j = 0; j < 4; ++j) {

@@ -22,6 +22,7 @@ struct GenFwdParams {
     GenericGeo geo;
     GenericDev d;
     int T;          // frames: 1 + (L + 2 (n_fft / 2) - n_fft) / hop
+    PoolRows pool;  // avse_mix_pooled: row indirection into a.speech / a.noise (speech_index == nullptr otherwise)
 };
 
 struct GenInvParams {
@@ -34,14 +35,14 @@ struct GenInvParams {
 };
 
 template <typename S>
-__device__ __forceinline__ float gen_sample(const S* p, int i, int L, int valid, int period = 0) {
+__device__ __forceinline__ float gen_sample(const S* p, int i, int L, int valid, int period = 0, int phase = 0) {
     // np.pad(y, n_fft // 2, mode='reflect') on the length-L (zero padded, dp:40) signal; period > 0: the signal is the
-    // periodic tiling p[i mod period] of a shorter noise file (dp:125-128)
+    // periodic tiling p[(phase + i) mod period] of a shorter noise file (dp:125-128; phase != 0: pooled pairs)
     i = i < 0 ? -i : i;
     i = i >= L ? 2 * (L - 1) - i : i;
     i = i < 0 ? 0 : i;
     if (p == nullptr || i >= valid) return 0.0f;
-    return (float)p[period > 0 ? i % period : i];
+    return (float)p[period > 0 ? (i + phase) % period : i];
 }
 
 // out[k1 + n1 k2] = sum_n in[n] W^{n k},  n = n2 a + c2.  `out` may alias `in`; tmp is scratch (shared memory).
@@ -108,29 +109,43 @@ __global__ void __launch_bounds__(GEN_THREADS) avse_generic_forward_kernel(const
     const int tid = threadIdx.x;
     const bool have_noise = A.noise != nullptr;
 
-    int vs = A.len_speech ? A.len_speech[u] : A.L;
-    int vn = A.len_noise ? A.len_noise[u] : vs;
-    vs = vs < 0 ? 0 : (vs < A.L ? vs : A.L);
-    vn = vn < 0 ? 0 : (vn < A.L ? vn : A.L);
+    int vs, vn, period, phase;
+    const S* sp;
+    const S* nz;
+    if (P.pool.speech_index != nullptr) {     // pooled pair (avse_mix_pooled): rows of the two pools, noise from its phase
+        const PoolRow r = pool_row(P.pool, u);
+        vs = r.ls < A.L ? r.ls : A.L;
+        vn = vs;
+        sp = reinterpret_cast<const S*>(A.speech) + r.s_off;
+        nz = reinterpret_cast<const S*>(A.noise) + r.n_off;
+        period = r.ln;
+        phase = r.off;
+    } else {
+        vs = A.len_speech ? A.len_speech[u] : A.L;
+        vn = A.len_noise ? A.len_noise[u] : vs;
+        vs = vs < 0 ? 0 : (vs < A.L ? vs : A.L);
+        vn = vn < 0 ? 0 : (vn < A.L ? vn : A.L);
+        period = (have_noise && A.noise_period) ? A.noise_period[u] : 0;
+        phase = 0;
+        sp = reinterpret_cast<const S*>(A.speech) + (size_t)u * A.in_stride;
+        nz = have_noise ? reinterpret_cast<const S*>(A.noise) + (size_t)u * A.in_stride : nullptr;
+    }
+    fit_noise_row(nz, period, phase, vn);          // a window that does not wrap is a contiguous row, read with no modulo
     // the whole SNR factor is applied after the transform: this path computes in float64, where the level equaliser of the
     // float32 kernels (avse_forward_args::equalizer) is not needed
     const float factor = have_noise ? (A.factor ? A.factor[u] : 1.0f) : 0.0f;
-    int period = (have_noise && A.noise_period) ? A.noise_period[u] : 0;
-    if (period <= 0 || period >= vn) period = 0;
-    const S* sp = reinterpret_cast<const S*>(A.speech) + (size_t)u * A.in_stride;
-    const S* nz = have_noise ? reinterpret_cast<const S*>(A.noise) + (size_t)u * A.in_stride : nullptr;
 
     if (tid < 3) { keys[tid] = (int)0x80000000; keys[3 + tid] = 0x7fffffff; }
     const int base = t * q.hop - N / 2;
     for (int n = tid; n < N; n += GEN_THREADS) {
         const double w = P.d.window[n];
-        X[n] = make_double2(gen_sample(sp, base + n, A.L, vs) * w, gen_sample(nz, base + n, A.L, vn, period) * w);
+        X[n] = make_double2(gen_sample(sp, base + n, A.L, vs) * w, gen_sample(nz, base + n, A.L, vn, period, phase) * w);
     }
     if (A.mixed_pcm != nullptr && have_noise) {     // this frame's own hop of s + f n (dp:133), zero padded / truncated to L
         float* pm = A.mixed_pcm + (size_t)u * A.pcm_stride;
         const int hi = (t + 1) * q.hop < A.L ? (t + 1) * q.hop : A.L;
         for (int i = t * q.hop + tid; i < hi; i += GEN_THREADS)
-            pm[i] = (i < vs ? (float)sp[i] : 0.0f) + factor * (i < vn ? (float)nz[period > 0 ? i % period : i] : 0.0f);
+            pm[i] = (i < vs ? (float)sp[i] : 0.0f) + factor * (i < vn ? (float)nz[period > 0 ? (i + phase) % period : i] : 0.0f);
     }
     __syncthreads();
     gen_dft(X, Y, X, W, N, q.n1, q.n2);
@@ -309,12 +324,12 @@ using namespace avse_gen;
 
 int avse_generic_frames(const avse::GenericGeo& q, int L) { return 1 + (L + 2 * (q.n_fft / 2) - q.n_fft) / q.hop; }
 
-int avse_generic_forward(avse_ctx* ctx, const avse_forward_args* args, void* stream) {
+int avse_generic_forward(avse_ctx* ctx, const avse_forward_args* args, const PoolRows* pool, void* stream) {
     const avse_forward_args& a = *args;
     const GenericGeo& q = ctx->gen.geo;
     if (!a.speech || !a.max_key) return avse_fail(AVSE_E_ARG, "avse_forward: speech and max_key are required");
     if (a.B <= 0 || a.L <= q.n_fft / 2) return avse_fail(AVSE_E_ARG, "avse_forward: need B > 0 and L > n_fft / 2 (reflect padding)");
-    if (!a.len_speech && a.in_stride < a.L) return avse_fail(AVSE_E_ARG, "avse_forward: in_stride < L needs len_speech");
+    if (!pool && !a.len_speech && a.in_stride < a.L) return avse_fail(AVSE_E_ARG, "avse_forward: in_stride < L needs len_speech");
     if (a.layout != AVSE_LAYOUT_SLICES && a.layout != AVSE_LAYOUT_SPEC) return avse_fail(AVSE_E_ARG, "avse_forward: bad layout");
     if (a.sample_format != AVSE_SAMPLE_F32 && a.sample_format != AVSE_SAMPLE_I16) return avse_fail(AVSE_E_ARG, "avse_forward: bad sample_format");
     GenFwdParams P;
@@ -322,6 +337,7 @@ int avse_generic_forward(avse_ctx* ctx, const avse_forward_args* args, void* str
     P.geo = q;
     P.d = ctx->gd;
     P.T = avse_generic_frames(q, a.L);
+    P.pool = pool ? *pool : PoolRows{};
     if (P.T < 1 || (long long)P.T * a.B > 0x7fffffffLL) return avse_fail(AVSE_E_ARG, "avse_forward: B * frames exceeds 2^31; split the batch");
     if (a.layout == AVSE_LAYOUT_SLICES) {
         if (a.n_slices < 0 || (long long)a.n_slices * q.spss > P.T) return avse_fail(AVSE_E_ARG, "avse_forward: n_slices exceeds int(T / spss) (dp:50)");

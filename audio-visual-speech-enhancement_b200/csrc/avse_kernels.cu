@@ -208,14 +208,33 @@ template <> struct Sample4<short> {
     }
 };
 
+// Float64 sums (sum x, sum x^2) of p[0, len) for the statistics pass: the vector part (vec: p is aligned) is split over the P
+// CTAs of the cluster, the scalar tail (the whole range when unaligned) goes to the last one.
+template <typename S>
+static __device__ __forceinline__ void range_sums(const S* p, int len, bool vec, int P, int part, double& x0, double& x1) {
+    const int n4 = vec ? (len >> 2) : 0;
+    const int per4 = (n4 + P - 1) / P;                       // this CTA's share of the vector part
+    const int lo4 = part * per4, hi4 = lo4 + per4 < n4 ? lo4 + per4 : n4;
+    for (int i = lo4 + threadIdx.x; i < hi4; i += blockDim.x) {
+        float v[4];
+        Sample4<S>::load(p, i, v);
+        x0 += (double)v[0] + (double)v[1] + (double)v[2] + (double)v[3];
+        x1 += (double)v[0] * v[0] + (double)v[1] * v[1] + (double)v[2] * v[2] + (double)v[3] * v[3];
+    }
+    if (part == P - 1)
+        for (int i = 4 * n4 + threadIdx.x; i < len; i += blockDim.x) { const double v = (double)p[i]; x0 += v; x1 += v * v; }
+}
+
 // One thread-block CLUSTER per utterance: the P CTAs of a cluster each reduce a contiguous part of the utterance and
 // rank 0 gathers their partial sums through distributed shared memory -- no scratch buffer, no second launch.  P = 1 for
 // the 3 s utterances of configs 1-3 (1 000 CTAs already fill the GPU); long-form audio (config 5: 64 x 60 s per GPU)
 // gets P = 8 so that all 148 SMs pull on HBM instead of 64.
+// pool.speech_index != nullptr (avse_mix_pooled): row u is the pooled pair pool_row(pool, u) (avse_common.h), its noise read
+// from its phase; otherwise row u of speech / noise, with the phase 0.
 template <typename S, bool CLUSTER>
 __global__ void __launch_bounds__(256) avse_snr_factor_kernel(const S* __restrict__ speech, const S* __restrict__ noise,
                                                               long long stride, const int* __restrict__ lengths,
-                                                              const int* __restrict__ noise_period, int L,
+                                                              const int* __restrict__ noise_period, int L, const PoolRows pool,
                                                               const float* __restrict__ snr_db, float* __restrict__ factor_out,
                                                               float* __restrict__ equalizer_out, int* __restrict__ max_key,
                                                               int* __restrict__ min_key) {
@@ -224,53 +243,48 @@ __global__ void __launch_bounds__(256) avse_snr_factor_kernel(const S* __restric
     const int P = CLUSTER ? (int)cluster.num_blocks() : 1;
     const int part = CLUSTER ? (int)cluster.block_rank() : 0;
     const int u = blockIdx.x / P;
-    int n = lengths ? lengths[u] : L;
-    n = n < 0 ? 0 : (n > L ? L : n);                          // never read past the row (stride >= L is checked by the launcher)
-    // dp:125-128: a noise file shorter than the speech is doubled until it covers it and then truncated, i.e. tiled
-    // periodically: noise[i] = nz[i mod Pn].  Its sums over [0, n) follow from one pass over the stored period:
-    // sample i < Pn occurs q + (i < rem) times, n = q Pn + rem.
-    int Pn = noise_period ? noise_period[u] : n;
-    Pn = (Pn <= 0 || Pn > n) ? n : Pn;
-    const int q = Pn > 0 ? n / Pn : 0, rem = Pn > 0 ? n - q * Pn : 0;
-    const S* s = speech + (size_t)u * stride;
-    const S* z = noise + (size_t)u * stride;
+    const S* s;
+    const S* z;
+    int n, Pn, off = 0;
+    bool bad = false;
+    if (pool.speech_index != nullptr) {
+        const PoolRow r = pool_row(pool, u);
+        s = speech + r.s_off;
+        z = noise + r.n_off;
+        n = r.ls;                                            // dp:130: the whole clip, before the pad / truncate to L
+        Pn = r.ln;
+        off = r.off;
+        bad = !r.ok;
+    } else {
+        n = lengths ? lengths[u] : L;
+        n = n < 0 ? 0 : (n > L ? L : n);                      // never read past the row (stride >= L is checked by the launcher)
+        // dp:125-128: a noise file shorter than the speech is doubled until it covers it and then truncated, i.e. tiled
+        // periodically: noise[i] = nz[i mod Pn]
+        Pn = noise_period ? noise_period[u] : n;
+        Pn = (Pn <= 0 || Pn > n) ? n : Pn;
+        s = speech + (size_t)u * stride;
+        z = noise + (size_t)u * stride;
+    }
+    const NoiseSpan span = noise_span(n, Pn, off);
     double a0 = 0.0, a1 = 0.0, b0 = 0.0, b1 = 0.0;
     constexpr size_t AL = sizeof(typename Sample4<S>::vec) - 1;
-    const int n4 = ((((size_t)s | (size_t)z) & AL) == 0) ? (n >> 2) : 0;
-    const int per4 = (n4 + P - 1) / P;                       // this CTA's share of the vector part
-    const int lo4 = part * per4, hi4 = lo4 + per4 < n4 ? lo4 + per4 : n4;
-    if (Pn == n) {
-        for (int i = lo4 + threadIdx.x; i < hi4; i += blockDim.x) {
-            float sv[4], zv[4];
-            Sample4<S>::load(s, i, sv);
-            Sample4<S>::load(z, i, zv);
-            a0 += (double)sv[0] + (double)sv[1] + (double)sv[2] + (double)sv[3];
-            a1 += (double)sv[0] * sv[0] + (double)sv[1] * sv[1] + (double)sv[2] * sv[2] + (double)sv[3] * sv[3];
-            b0 += (double)zv[0] + (double)zv[1] + (double)zv[2] + (double)zv[3];
-            b1 += (double)zv[0] * zv[0] + (double)zv[1] * zv[1] + (double)zv[2] * zv[2] + (double)zv[3] * zv[3];
-        }
-        if (part == P - 1)                                   // scalar tail (and the whole signal when it is unaligned)
-            for (int i = 4 * n4 + threadIdx.x; i < n; i += blockDim.x) {
-                const double sv = (double)s[i], zv = (double)z[i];
-                a0 += sv; a1 += sv * sv; b0 += zv; b1 += zv * zv;
-            }
+    // identity rows keep the joint alignment test of the two rows (the summation order of the existing entry points)
+    const bool vec_s = ((((size_t)s | (pool.speech_index ? 0 : (size_t)z)) & AL) == 0);
+    range_sums(s, n, vec_s, P, part, a0, a1);
+    if (!span.periodic) {
+        const S* z0 = z + off;
+        range_sums(z0, span.len0, pool.speech_index ? (((size_t)z0 & AL) == 0) : vec_s, P, part, b0, b1);
+        if (span.len1 > 0) range_sums(z, span.len1, ((size_t)z & AL) == 0, P, part, b0, b1);     // the window wraps
     } else {
-        // tiled noise (rare: the noise file is shorter than the utterance): speech over [0, n), noise over its period
-        for (int i = lo4 + threadIdx.x; i < hi4; i += blockDim.x) {
-            float sv[4];
-            Sample4<S>::load(s, i, sv);
-            a0 += (double)sv[0] + (double)sv[1] + (double)sv[2] + (double)sv[3];
-            a1 += (double)sv[0] * sv[0] + (double)sv[1] * sv[1] + (double)sv[2] * sv[2] + (double)sv[3] * sv[3];
-        }
-        if (part == P - 1)
-            for (int i = 4 * n4 + threadIdx.x; i < n; i += blockDim.x) { const double sv = (double)s[i]; a0 += sv; a1 += sv * sv; }
+        // tiled noise (the noise file is shorter than the utterance): one weighted pass over its period
         const int perp = (Pn + P - 1) / P;
         const int lop = part * perp, hip = lop + perp < Pn ? lop + perp : Pn;
         for (int i = lop + threadIdx.x; i < hip; i += blockDim.x) {
-            const double zv = (double)z[i], w = (double)(q + (i < rem ? 1 : 0));
+            const double zv = (double)z[i], w = (double)noise_weight(span, i, Pn, off);
             b0 += w * zv; b1 += w * zv * zv;
         }
     }
+    if (bad && part == 0 && threadIdx.x == 0) atomicExch(pool.bad_row_flag, 1);
     __shared__ double red[4][8];
     __shared__ double partial[4];
 #pragma unroll
@@ -318,10 +332,10 @@ __global__ void __launch_bounds__(256) avse_snr_factor_kernel(const S* __restric
 
 template <typename S>
 static cudaError_t launch_snr_factor(int B, int P, cudaStream_t st, const S* speech, const S* noise, long long stride, const int* lengths,
-                                     const int* noise_period, int L, const float* snr_db, float* factor_out, float* equalizer_out,
-                                     int* max_key, int* min_key) {
+                                     const int* noise_period, int L, const PoolRows& pool, const float* snr_db, float* factor_out,
+                                     float* equalizer_out, int* max_key, int* min_key) {
     if (P == 1) {       // plain launch: cluster launches carry extra scheduling constraints
-        avse_snr_factor_kernel<S, false><<<B, 256, 0, st>>>(speech, noise, stride, lengths, noise_period, L, snr_db, factor_out,
+        avse_snr_factor_kernel<S, false><<<B, 256, 0, st>>>(speech, noise, stride, lengths, noise_period, L, pool, snr_db, factor_out,
                                                             equalizer_out, max_key, min_key);
         return cudaGetLastError();
     }
@@ -337,8 +351,29 @@ static cudaError_t launch_snr_factor(int B, int P, cudaStream_t st, const S* spe
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, avse_snr_factor_kernel<S, true>, speech, noise, stride, lengths, noise_period, L, snr_db, factor_out,
+    return cudaLaunchKernelEx(&cfg, avse_snr_factor_kernel<S, true>, speech, noise, stride, lengths, noise_period, L, pool, snr_db, factor_out,
                               equalizer_out, max_key, min_key);
+}
+
+// Statistics launch shared by avse_snr_factor (identity rows: pool.speech_index == nullptr) and avse_mix_pooled.  `L` sizes the
+// cluster: the longest row the pass may read.
+static int snr_factor_launch(avse_ctx* ctx, const void* speech, const void* noise, int sample_format, long long stride, const int* lengths,
+                             const int* noise_period, int B, int L, const PoolRows& pool, const float* snr_db, float* factor_out,
+                             float* equalizer_out, int* max_key, int* min_key, void* stream) {
+    // cluster size: enough CTAs to occupy every SM a few times over, each with >= 64 K samples, at most 8 (portable limit)
+    int P = 1;
+    while (P < 8 && (long long)B * P < 4LL * ctx->num_sms && L / (2 * P) >= 65536) P *= 2;
+    cudaError_t e;
+    if (sample_format == AVSE_SAMPLE_F32)
+        e = launch_snr_factor<float>(B, P, (cudaStream_t)stream, (const float*)speech, (const float*)noise, stride, lengths, noise_period, L,
+                                     pool, snr_db, factor_out, equalizer_out, max_key, min_key);
+    else if (sample_format == AVSE_SAMPLE_I16)
+        e = launch_snr_factor<short>(B, P, (cudaStream_t)stream, (const short*)speech, (const short*)noise, stride, lengths, noise_period, L,
+                                     pool, snr_db, factor_out, equalizer_out, max_key, min_key);
+    else return avse_fail(AVSE_E_ARG, "avse_snr_factor: bad sample_format");
+    if (e != cudaSuccess) return avse_cuda_fail(e, "avse_snr_factor launch");
+    CUDA_TRY(cudaGetLastError());
+    return 0;
 }
 
 extern "C" int avse_snr_factor(avse_ctx* ctx, const void* speech, const void* noise, int sample_format, long long stride,
@@ -346,20 +381,9 @@ extern "C" int avse_snr_factor(avse_ctx* ctx, const void* speech, const void* no
                                float* equalizer_out, int* max_key, int* min_key, void* stream) {
     if (!ctx || !speech || !noise || !factor_out) return avse_fail(AVSE_E_ARG, "avse_snr_factor: NULL argument");
     if (B <= 0 || L <= 0 || stride < L) return avse_fail(AVSE_E_ARG, "avse_snr_factor: bad sizes");
-    // cluster size: enough CTAs to occupy every SM a few times over, each with >= 64 K samples, at most 8 (portable limit)
-    int P = 1;
-    while (P < 8 && (long long)B * P < 4LL * ctx->num_sms && L / (2 * P) >= 65536) P *= 2;
-    cudaError_t e;
-    if (sample_format == AVSE_SAMPLE_F32)
-        e = launch_snr_factor<float>(B, P, (cudaStream_t)stream, (const float*)speech, (const float*)noise, stride, lengths, noise_period, L,
-                                     snr_db, factor_out, equalizer_out, max_key, min_key);
-    else if (sample_format == AVSE_SAMPLE_I16)
-        e = launch_snr_factor<short>(B, P, (cudaStream_t)stream, (const short*)speech, (const short*)noise, stride, lengths, noise_period, L,
-                                     snr_db, factor_out, equalizer_out, max_key, min_key);
-    else return avse_fail(AVSE_E_ARG, "avse_snr_factor: bad sample_format");
-    if (e != cudaSuccess) return avse_cuda_fail(e, "avse_snr_factor launch");
-    CUDA_TRY(cudaGetLastError());
-    return 0;
+    const PoolRows identity = {};
+    return snr_factor_launch(ctx, speech, noise, sample_format, stride, lengths, noise_period, B, L, identity, snr_db, factor_out,
+                             equalizer_out, max_key, min_key, stream);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -411,6 +435,7 @@ struct FwdParams {
     int total_tiles;  // B * G
     int per_warp;     // tiles per warp (contiguous range): the 2-frame kernel
     WarpSplit split;  // F4 kernel: balanced contiguous ranges (avse_common.h)
+    PoolRows pool;    // avse_mix_pooled: row indirection into the speech / noise pools (a.speech / a.noise); speech_index == nullptr otherwise
 };
 
 // SCAN = true: fused post+mel scan (tables with scan_ok); false: generic banded gather.
@@ -452,7 +477,9 @@ __global__ void __launch_bounds__(FWD_THREADS, FWD_CTAS) avse_forward_kernel(con
 
     float mx[3] = {neg_inf(), neg_inf(), neg_inf()};
     float factor = 0.0f, gain = 0.0f;
-    int vs = 0, vn = 0, period = 0;
+    int vs = 0, vn = 0, period = 0, phase = 0;
+    const float* sp_row = nullptr;
+    const float* nz_row = nullptr;
     bool fresh = true;
 
     auto flush_max = [&](int uu) {
@@ -470,19 +497,32 @@ __global__ void __launch_bounds__(FWD_THREADS, FWD_CTAS) avse_forward_kernel(con
     for (int it = 0; it < n_tiles; ++it) {
         if (fresh) {
             fresh = false;
-            vs = A.len_speech ? A.len_speech[u] : A.L;
-            vn = A.len_noise ? A.len_noise[u] : vs;
-            vs = vs < 0 ? 0 : (vs < A.L ? vs : A.L);
-            vn = vn < 0 ? 0 : (vn < A.L ? vn : A.L);
+            if (P.pool.speech_index != nullptr) {           // pooled pair (avse_mix_pooled): always a pair batch
+                const PoolRow r = pool_row(P.pool, u);
+                vs = r.ls < A.L ? r.ls : A.L;
+                vn = vs;
+                sp_row = static_cast<const float*>(A.speech) + r.s_off;
+                nz_row = static_cast<const float*>(A.noise) + r.n_off;
+                period = r.ln;
+                phase = r.off;
+            } else {
+                vs = A.len_speech ? A.len_speech[u] : A.L;
+                vn = A.len_noise ? A.len_noise[u] : vs;
+                vs = vs < 0 ? 0 : (vs < A.L ? vs : A.L);
+                vn = vn < 0 ? 0 : (vn < A.L ? vn : A.L);
+                sp_row = static_cast<const float*>(A.speech) + (size_t)u * A.in_stride;
+                nz_row = have_noise ? static_cast<const float*>(A.noise) + (size_t)u * A.in_stride : nullptr;
+                period = (have_noise && A.noise_period) ? A.noise_period[u] : 0;
+                phase = 0;
+            }
+            fit_noise_row(nz_row, period, phase, vn);        // a window that does not wrap is a contiguous row
             const MixGain mg = mix_gain(A, u);
             factor = have_noise ? mg.resid : 0.0f;
             gain = have_noise ? mg.gain : 0.0f;
-            period = (have_noise && A.noise_period) ? A.noise_period[u] : 0;
-            if (period <= 0 || period >= vn) period = 0;      // the stored noise already covers [0, vn)
         }
         FwdTile tl;
-        tl.sp = static_cast<const float*>(A.speech) + (size_t)u * A.in_stride;
-        tl.nz = have_noise ? static_cast<const float*>(A.noise) + (size_t)u * A.in_stride : nullptr;
+        tl.sp = sp_row;
+        tl.nz = nz_row;
         tl.L = A.L;
         tl.valid_s = vs;
         tl.valid_n = vn;
@@ -492,6 +532,7 @@ __global__ void __launch_bounds__(FWD_THREADS, FWD_CTAS) avse_forward_kernel(con
         tl.factor = factor;
         tl.gain = gain;
         tl.period_n = period;
+        tl.phase_n = phase;
         tl.mixed_pcm = A.mixed_pcm ? A.mixed_pcm + (size_t)u * A.pcm_stride : nullptr;
 
         // ---- pass 1 ----
@@ -595,8 +636,10 @@ constexpr int F4_SM_MIN = F4_SM_LOC + NMEL * 4;                // [warps][3][32]
 #define AVSE_F4_PTR_SLOT 1         // 1: the utterance's output row pointers live in the per-warp slot (written once per utterance)
 #endif
 constexpr int F4_UTT_F = AVSE_F4_PTR_SLOT ? 12 : 2;            // per parity: gain, noise period [, 4 output row pointers, 2 pad]
-constexpr int F4_SM_UTT = F4_SM_MIN + F4_WARPS * 96;           // [warps][2][F4_UTT_F] per-utterance values, see the kernel
-constexpr int F4_SMEM_F = F4_SM_UTT + F4_WARPS * 2 * F4_UTT_F;
+constexpr int F4_UTT_TILED_F = F4_UTT_F + 6;                   // TILED: + input row pointers (speech, noise), noise phase, 1 pad
+constexpr int F4_SM_UTT = F4_SM_MIN + F4_WARPS * 96;           // [warps][2][F4_UTT_F or F4_UTT_TILED_F] per-utterance values, see the kernel
+constexpr int F4_SMEM_F = F4_SM_UTT + F4_WARPS * 2 * F4_UTT_TILED_F;
+static_assert((F4_UTT_F % 2) == 0 && (F4_UTT_TILED_F % 2) == 0, "8-byte aligned pointer slots");
 constexpr int F4_SMEM_BYTES = F4_SMEM_F * 4;
 static_assert((F4_SM_TW % 2) == 0 && (F4_SM_SCANW % 2) == 0 && (F4_SM_LOC % 4) == 0 && (F4_SM_UTT % 4) == 0, "table alignment");
 static_assert(F4_SMEM_BYTES + 1024 <= 232448, "F4 shared memory must fit in one SM");
@@ -626,9 +669,12 @@ __device__ __noinline__ void f4_fill_tables(float* smem, float* frames, const fl
     table_put(smem + F4_SM_LOC, tid, r_loc);
 }
 
-// TILED: the batch carries per-utterance noise periods (avse_forward_args::noise_period, dp:125-128).  A separate
-// instantiation, because this kernel sits on the 255-register / 32 KB instruction-cache cliff: with the period logic
-// compiled into the common kernel, batches that do not use it ran 4.5 % slower (profiles/README.md, round 2).
+// TILED: the batch carries per-utterance noise periods (avse_forward_args::noise_period, dp:125-128), or it is a pooled batch
+// (avse_mix_pooled: per-row speech / noise clips of two pools, the noise read from a phase).  load_utt resolves, once per
+// utterance, the two input row pointers, the noise period and the phase into the warp's slot; identity rows with phase 0 are
+// the noise_period case.  A separate instantiation, because this kernel sits on the 255-register / 32 KB instruction-cache
+// cliff: with the period logic compiled into the common kernel, batches that do not use it ran 4.5 % slower
+// (profiles/README.md, round 2).
 template <typename S, bool TILED, bool PAD>
 __global__ void __launch_bounds__(F4_THREADS, 1) avse_forward4_kernel(const __grid_constant__ FwdParams P) {
     extern __shared__ __align__(16) float smem[];
@@ -670,7 +716,8 @@ __global__ void __launch_bounds__(F4_THREADS, 1) avse_forward4_kernel(const __gr
     int vs = 0, vn = 0;
     // the level-equaliser gain (and the noise period) are needed once per tile, at the top of pass 1: they live in a
     // per-warp shared-memory slot, double-buffered by the utterance's parity, instead of in loop-carried registers
-    float* utt_sm = smem + F4_SM_UTT + warp * (2 * F4_UTT_F);
+    constexpr int UF = TILED ? F4_UTT_TILED_F : F4_UTT_F;         // slot floats per parity
+    float* utt_sm = smem + F4_SM_UTT + warp * (2 * UF);
     const S* in_speech = reinterpret_cast<const S*>(A.speech);
     const S* in_noise = reinterpret_cast<const S*>(A.noise);
     constexpr int LINE = 128 / (int)sizeof(S);        // samples per 128-byte line
@@ -693,7 +740,7 @@ __global__ void __launch_bounds__(F4_THREADS, 1) avse_forward4_kernel(const __gr
         }
     };
 
-    auto prefetch_ahead = [&](int it, int u, int g) {
+    auto prefetch_ahead = [&](int it, int u, int g, const FwdTileT<S>& tc) {
 #if AVSE_F4_PREFETCH > 0
         // L2 prefetch of the samples this warp first touches AVSE_F4_PREFETCH groups from now (own tiles only)
         if (it + AVSE_F4_PREFETCH < n_tiles) {
@@ -702,7 +749,12 @@ __global__ void __launch_bounds__(F4_THREADS, 1) avse_forward4_kernel(const __gr
             const int lo = g2 == 0 ? 0 : g2 * (F4 * HOP) + HOP;      // first sample not covered by group g2 - 1
             const int hi = g2 * (F4 * HOP) + (NFFT + HOP);           // window end of group g2 (exclusive)
             const int i0 = (lo & ~(LINE - 1)) + LINE * lane;         // one 128-byte line per lane
-            if (i0 < hi && i0 < A.L && i0 < A.in_stride && lane < 22) {
+            if (TILED) {      // rows resolved per utterance: this utterance's own rows only, a tiled noise is not prefetched
+                if (u2 == u && i0 < hi && i0 < tc.valid_s && lane < 22) {
+                    asm volatile("prefetch.global.L2 [%0];" ::"l"(tc.sp + i0));
+                    if (tc.period_n == 0 && i0 < tc.valid_n) asm volatile("prefetch.global.L2 [%0];" ::"l"(tc.nz + i0));
+                }
+            } else if (i0 < hi && i0 < A.L && i0 < A.in_stride && lane < 22) {
                 const size_t o = (size_t)u2 * A.in_stride + i0;
                 asm volatile("prefetch.global.L2 [%0];" ::"l"(in_speech + o));
                 asm volatile("prefetch.global.L2 [%0];" ::"l"(in_noise + o));
@@ -719,10 +771,10 @@ __global__ void __launch_bounds__(F4_THREADS, 1) avse_forward4_kernel(const __gr
         ovn = ovn < 0 ? 0 : (ovn < A.L ? ovn : A.L);
         const MixGain mg = mix_gain(A, uu);
         of = mg.resid;
-        utt_sm[F4_UTT_F * (uu & 1)] = mg.gain;                // every lane writes the same value
+        utt_sm[UF * (uu & 1)] = mg.gain;                      // every lane writes the same value
 #if AVSE_F4_PTR_SLOT
         {   // this utterance's output rows (null stays null): read back once per tile instead of 64-bit multiplies + null checks
-            float** ps = reinterpret_cast<float**>(utt_sm + F4_UTT_F * (uu & 1) + 2);
+            float** ps = reinterpret_cast<float**>(utt_sm + UF * (uu & 1) + 2);
             ps[0] = A.out_speech ? A.out_speech + (size_t)uu * A.out_stride : nullptr;
             ps[1] = A.out_noise ? A.out_noise + (size_t)uu * A.out_stride : nullptr;
             ps[2] = A.out_mixed ? A.out_mixed + (size_t)uu * A.out_stride : nullptr;
@@ -730,15 +782,42 @@ __global__ void __launch_bounds__(F4_THREADS, 1) avse_forward4_kernel(const __gr
         }
 #endif
         if (TILED) {
-            int period = A.noise_period[uu];
-            if (period <= 0 || period >= ovn) period = 0;     // the stored noise already covers [0, vn)
-            reinterpret_cast<int*>(utt_sm)[F4_UTT_F * (uu & 1) + 1] = period;
+            const S* sp;
+            const S* nz;
+            int period, phase;
+            if (P.pool.speech_index != nullptr) {             // pooled pair: rows of the two pools, noise from its phase
+                const PoolRow r = pool_row(P.pool, uu);
+                ovs = r.ls < A.L ? r.ls : A.L;
+                ovn = ovs;
+                sp = in_speech + r.s_off;
+                nz = in_noise + r.n_off;
+                period = r.ln;
+                phase = r.off;
+            } else {
+                sp = in_speech + (size_t)uu * A.in_stride;
+                nz = in_noise + (size_t)uu * A.in_stride;
+                period = A.noise_period[uu];
+                phase = 0;
+            }
+            fit_noise_row(nz, period, phase, ovn);            // the stored noise already covers the window: no modulo
+            int* si = reinterpret_cast<int*>(utt_sm + UF * (uu & 1));
+            si[1] = period;
+            si[F4_UTT_F + 4] = phase;
+            const S** pi = reinterpret_cast<const S**>(utt_sm + UF * (uu & 1) + F4_UTT_F);
+            pi[0] = sp;
+            pi[1] = nz;
         }
     };
     auto make_tile = [&](int uu, int gg, int tvs, int tvn, float tf) {
         FwdTileT<S> t;
-        t.sp = in_speech + (size_t)uu * A.in_stride;      // (the INPUT row pointers through the slot too: 3 % slower -- they feed the
-        t.nz = in_noise + (size_t)uu * A.in_stride;       //  address generation of the software-pipelined loads)
+        if (TILED) {
+            const S* const* pi = reinterpret_cast<const S* const*>(utt_sm + UF * (uu & 1) + F4_UTT_F);
+            t.sp = pi[0];
+            t.nz = pi[1];
+        } else {
+            t.sp = in_speech + (size_t)uu * A.in_stride;  // (the INPUT row pointers through the slot too: 3 % slower -- they feed the
+            t.nz = in_noise + (size_t)uu * A.in_stride;   //  address generation of the software-pipelined loads)
+        }
         t.L = A.L;
         t.valid_s = tvs;
         t.valid_n = tvn;
@@ -747,9 +826,10 @@ __global__ void __launch_bounds__(F4_THREADS, 1) avse_forward4_kernel(const __gr
         t.t0 = gg * F4;
         t.factor = tf;
         t.gain = 0.0f;            // read from the slot at the top of pass 1
-        t.period_n = TILED ? reinterpret_cast<const int*>(utt_sm)[F4_UTT_F * (uu & 1) + 1] : 0;
+        t.period_n = TILED ? reinterpret_cast<const int*>(utt_sm)[UF * (uu & 1) + 1] : 0;
+        t.phase_n = TILED ? reinterpret_cast<const int*>(utt_sm)[UF * (uu & 1) + F4_UTT_F + 4] : 0;
 #if AVSE_F4_PTR_SLOT
-        t.mixed_pcm = reinterpret_cast<float* const*>(utt_sm + F4_UTT_F * (uu & 1) + 2)[3];
+        t.mixed_pcm = reinterpret_cast<float* const*>(utt_sm + UF * (uu & 1) + 2)[3];
 #else
         t.mixed_pcm = A.mixed_pcm ? A.mixed_pcm + (size_t)uu * A.pcm_stride : nullptr;
 #endif
@@ -770,9 +850,9 @@ __global__ void __launch_bounds__(F4_THREADS, 1) avse_forward4_kernel(const __gr
     }
 #pragma unroll 1
     for (int it = 0; it < n_tiles; ++it) {
-        prefetch_ahead(it, u, g);
+        prefetch_ahead(it, u, g, tl);
         // ---- pass 1 ----
-        tl.gain = utt_sm[F4_UTT_F * (u & 1)];
+        tl.gain = utt_sm[UF * (u & 1)];
         if (reflect) {                       // mirrored loads, interior arithmetic; this group's PCM stores need their bounds check
             stage4_store_pcm_guarded(tl, lane, rs, rn, ts, tn);
             tl.mixed_pcm = nullptr;
@@ -826,7 +906,7 @@ __global__ void __launch_bounds__(F4_THREADS, 1) avse_forward4_kernel(const __gr
         {
             FwdOut out;
 #if AVSE_F4_PTR_SLOT
-            float* const* ps = reinterpret_cast<float* const*>(utt_sm + F4_UTT_F * (u & 1) + 2);
+            float* const* ps = reinterpret_cast<float* const*>(utt_sm + UF * (u & 1) + 2);
             out.dst[0] = ps[0]; out.dst[1] = ps[1]; out.dst[2] = ps[2];
 #else
             out.dst[0] = A.out_speech ? A.out_speech + (size_t)u * A.out_stride : nullptr;
@@ -856,16 +936,13 @@ __global__ void __launch_bounds__(F4_THREADS, 1) avse_forward4_kernel(const __gr
 
 __global__ void avse_reset_max_kernel(int* __restrict__ max_key, int* __restrict__ min_key, int n, int min_value);
 
-extern "C" int avse_forward(avse_ctx* ctx, const avse_forward_args* args, void* stream) {
-    if (!ctx || !args) return avse_fail(AVSE_E_ARG, "avse_forward: NULL argument");
-    if (ctx->generic) return avse_generic_forward(ctx, args, stream);
-    const avse_forward_args& a = *args;
-    if (!a.speech || !a.max_key) return avse_fail(AVSE_E_ARG, "avse_forward: speech and max_key are required");
+// The forward launch of avse_forward (pool.speech_index == nullptr) and avse_mix_pooled (specialised geometry).
+static int forward_launch(avse_ctx* ctx, const avse_forward_args& a, const PoolRows& pool, void* stream) {
     if (a.B <= 0 || a.L <= HALF) return avse_fail(AVSE_E_ARG, "avse_forward: need B > 0 and L > 320 (reflect padding)");
-    if (!a.len_speech && a.in_stride < a.L) return avse_fail(AVSE_E_ARG, "avse_forward: in_stride < L needs len_speech");
     if (a.layout != AVSE_LAYOUT_SLICES && a.layout != AVSE_LAYOUT_SPEC) return avse_fail(AVSE_E_ARG, "avse_forward: bad layout");
     FwdParams P;
     P.a = a;
+    P.pool = pool;
     P.tb = ctx->fwd;
     P.T = 1 + a.L / HOP;
     P.G = (P.T + FPG - 1) / FPG;
@@ -912,7 +989,7 @@ extern "C" int avse_forward(avse_ctx* ctx, const avse_forward_args* args, void* 
         P.total_tiles = (int)total4;
         P.per_warp = (int)((total4 + nwarps4 - 1) / nwarps4);
         P.split = make_warp_split(total4, blocks4, F4_WARPS);
-        const bool tiled = a.noise_period != nullptr;
+        const bool tiled = a.noise_period != nullptr || pool.speech_index != nullptr;
         // PAD: the batch carries per-utterance lengths, so rows may be zero-padded (see avse_fwd4_stages.cuh); never together with TILED
         const bool pad = !tiled && (a.len_speech != nullptr || a.len_noise != nullptr);
         const cudaStream_t st4 = (cudaStream_t)stream;
@@ -944,6 +1021,17 @@ extern "C" int avse_forward(avse_ctx* ctx, const avse_forward_args* args, void* 
         CUDA_TRY(cudaGetLastError());
     }
     return 0;
+}
+
+extern "C" int avse_forward(avse_ctx* ctx, const avse_forward_args* args, void* stream) {
+    if (!ctx || !args) return avse_fail(AVSE_E_ARG, "avse_forward: NULL argument");
+    if (ctx->generic) return avse_generic_forward(ctx, args, nullptr, stream);
+    const avse_forward_args& a = *args;
+    if (!a.speech || !a.max_key) return avse_fail(AVSE_E_ARG, "avse_forward: speech and max_key are required");
+    if (a.B <= 0 || a.L <= HALF) return avse_fail(AVSE_E_ARG, "avse_forward: need B > 0 and L > 320 (reflect padding)");
+    if (!a.len_speech && a.in_stride < a.L) return avse_fail(AVSE_E_ARG, "avse_forward: in_stride < L needs len_speech");
+    const PoolRows identity = {};
+    return forward_launch(ctx, a, identity, stream);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1091,6 +1179,77 @@ extern "C" int avse_max_db(avse_ctx* ctx, const int* max_key, int n, float* out_
     avse_max_db_kernel<<<(n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(max_key, n, out_db);
     CUDA_TRY(cudaGetLastError());
     return 0;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Pooled pairs: preprocess_audio_pair (dp:119-139) of (speech clip speech_index[b], noise clip noise_index[b] read from
+// noise_offset[b] on) for every output row b, straight from two device-resident clip pools (see include/avse_b200.h).
+// Three launches on `stream`: the statistics pass (which also flags invalid rows), the forward kernel, the top_db floor.
+// ---------------------------------------------------------------------------------------------
+extern "C" int avse_mix_pooled(avse_ctx* ctx, const avse_pool_mix_args* args, void* stream) {
+    if (!ctx || !args) return avse_fail(AVSE_E_ARG, "avse_mix_pooled: NULL argument");
+    const avse_pool_mix_args& m = *args;
+    if (!m.speech_pool || !m.noise_pool || !m.speech_len || !m.noise_len || !m.speech_index || !m.noise_index)
+        return avse_fail(AVSE_E_ARG, "avse_mix_pooled: pools, clip lengths and row indices are required");
+    if (!m.out_speech || !m.out_noise || !m.out_mixed || !m.factor_out || !m.max_key || !m.bad_row_flag)
+        return avse_fail(AVSE_E_ARG, "avse_mix_pooled: the three slice outputs, factor_out, max_key and bad_row_flag are required");
+    if (m.n_speech <= 0 || m.n_noise <= 0 || m.speech_stride <= 0 || m.noise_stride <= 0)
+        return avse_fail(AVSE_E_ARG, "avse_mix_pooled: empty pool (n_speech, n_noise and both strides must be > 0)");
+    if (m.B <= 0 || m.n_slices <= 0) return avse_fail(AVSE_E_ARG, "avse_mix_pooled: need B > 0 and n_slices > 0");
+    if (m.sample_format != AVSE_SAMPLE_F32 && m.sample_format != AVSE_SAMPLE_I16) return avse_fail(AVSE_E_ARG, "avse_mix_pooled: bad sample_format");
+    PoolRows pool;
+    pool.speech_index = m.speech_index;
+    pool.noise_index = m.noise_index;
+    pool.noise_offset = m.noise_offset;
+    pool.speech_len = m.speech_len;
+    pool.noise_len = m.noise_len;
+    pool.speech_stride = m.speech_stride;
+    pool.noise_stride = m.noise_stride;
+    pool.n_speech = m.n_speech;
+    pool.n_noise = m.n_noise;
+    pool.bad_row_flag = m.bad_row_flag;
+    avse_forward_args a = {};
+    a.speech = m.speech_pool;
+    a.noise = m.noise_pool;
+    a.factor = m.factor_out;
+    a.B = m.B;
+    a.L = m.L;
+    a.layout = AVSE_LAYOUT_SLICES;
+    a.n_slices = m.n_slices;
+    a.out_speech = m.out_speech;
+    a.out_noise = m.out_noise;
+    a.out_mixed = m.out_mixed;
+    a.out_stride = m.out_stride;
+    a.mixed_pcm = m.mixed_pcm;
+    a.pcm_stride = m.pcm_stride;
+    a.max_key = m.max_key;
+    a.min_key = m.min_key;
+    a.sample_format = m.sample_format;
+    a.equalizer = m.equalizer_out;
+    // refuse what the forward pass would refuse before the statistics pass is enqueued
+    const int half = ctx->generic ? ctx->n_fft / 2 : HALF;
+    if (m.L <= half) return avse_fail(AVSE_E_ARG, "avse_mix_pooled: need L > n_fft / 2 (reflect padding)");
+    const int T = ctx->generic ? avse_generic_frames(ctx->gen.geo, m.L) : 1 + m.L / HOP;
+    if ((long long)m.n_slices * ctx->spss > T) return avse_fail(AVSE_E_ARG, "avse_mix_pooled: n_slices exceeds int(T / spss) (dp:50)");
+    const long long n_per_utt = (long long)m.n_slices * ctx->n_mels * ctx->spss;
+    if (m.out_stride < n_per_utt) return avse_fail(AVSE_E_ARG, "avse_mix_pooled: out_stride too small");
+    float* outs[3] = {m.out_speech, m.out_noise, m.out_mixed};
+    for (int s = 0; s < 3; ++s)
+        if (((size_t)outs[s] & 15) || (m.out_stride & 3)) return avse_fail(AVSE_E_ARG, "avse_mix_pooled: outputs must be 16-byte aligned with out_stride % 4 == 0");
+    if (m.mixed_pcm && m.pcm_stride < m.L) return avse_fail(AVSE_E_ARG, "avse_mix_pooled: pcm_stride < L");
+    if (m.sample_format == AVSE_SAMPLE_I16 && !ctx->generic && !ctx->f4_tables)
+        return avse_fail(AVSE_E_ARG, "avse_mix_pooled: int16 samples need the standard 2-tap filterbank; convert the pools to float32 first");
+    int dev = 0;
+    CUDA_TRY(cudaGetDevice(&dev));
+    if (dev != ctx->device) return avse_fail(AVSE_E_ARG, "avse_mix_pooled: current device differs from the context's device");
+
+    const int longest = m.speech_stride < 0x7fffffffLL ? (int)m.speech_stride : 0x7fffffff;     // sizes the statistics clusters
+    int rc = snr_factor_launch(ctx, m.speech_pool, m.noise_pool, m.sample_format, 0, nullptr, nullptr, m.B, longest, pool, m.snr_db,
+                               m.factor_out, m.equalizer_out, m.max_key, m.min_key, stream);
+    if (rc != 0) return rc;
+    rc = ctx->generic ? avse_generic_forward(ctx, &a, &pool, stream) : forward_launch(ctx, a, pool, stream);
+    if (rc != 0) return rc;
+    return avse_floor_inplace3(ctx, m.out_speech, m.out_noise, m.out_mixed, m.out_stride, n_per_utt, m.B, m.max_key, m.min_key, stream);
 }
 
 // ---------------------------------------------------------------------------------------------

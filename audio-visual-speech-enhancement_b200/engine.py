@@ -14,7 +14,7 @@ import numpy as np
 import torch
 
 from . import _native
-from ._native import ForwardArgs, InverseArgs, check
+from ._native import ForwardArgs, InverseArgs, PoolMixArgs, check
 
 N_FFT, HOP, N_BINS, N_MELS, SPSS = 640, 160, 321, 80, 20
 LAYOUT_SLICES, LAYOUT_SPEC = 0, 1
@@ -308,6 +308,78 @@ class SpectralEngine(object):
         if info is not None:        # side data for callers that need it: the SNR factors (dp:130) and the dB extrema
             info["factor"], info["keys"] = factor, max_key
         return res["mixed"], res["speech"], res["noise"], res["mixed_pcm"]
+
+    @_on_device
+    def mix_pools(self, speech_pool, speech_lengths, noise_pool, noise_lengths, speech_index, noise_index, n_video_slices,
+                  noise_offset=None, snr_db=None, out=None, info=None, check=True):
+        """preprocess_audio_pair (dp:119-139) of pairings drawn from two device-resident clip pools (avse_mix_pooled).
+
+        speech_pool [Ns, >= max clip] / noise_pool [Nn, >= max clip]: float32, or int16 for both (raw WAV samples, decoded in
+        the kernels); speech_lengths [Ns] / noise_lengths [Nn] int32 clip lengths (see pack_clips).  Row b mixes speech clip
+        speech_index[b] with noise clip noise_index[b] read from sample noise_offset[b] on and wrapped around its length:
+        n[i] = z[(off + i) mod Ln] (off = 0, the default, is the reference's tile-or-truncate rule, dp:125-128), at snr_db[b]
+        (default 0 dB, dp:130).  No pairing is materialised.
+        Returns (mixed, speech, noise, mixed_pcm) shaped like preprocess_pairs: [B, n, 80, 20] x3 and [B, L],
+        n = min(n_video_slices, int(T/20)).
+        A row with an index out of range or an offset outside [0, Ln) is invalid: it is processed as an empty pair (every slice
+        at -100 dB, PCM zeros).  check=True reads the device flag back (one synchronisation) and raises IndexError; check=False
+        stays asynchronous.  out: dict whose tensors are re-used from call to call (like preprocess_pairs / HostPipeline).
+        info: optional dict that receives `factor` [B], the dB `keys` (DbKeys) and `valid` [B] bool = row valid and factor
+        finite (a silent noise window gives inf / nan like numpy)."""
+        i16 = speech_pool.dtype == torch.int16 and noise_pool.dtype == torch.int16
+        sp, nz = self._as_batch(speech_pool, i16), self._as_batch(noise_pool, i16)
+        dev = self.device
+        slen = torch.as_tensor(speech_lengths, device=dev).to(torch.int32).contiguous()
+        nlen = torch.as_tensor(noise_lengths, device=dev).to(torch.int32).contiguous()
+        assert slen.numel() == sp.shape[0] and nlen.numel() == nz.shape[0], "one length per pool clip"
+        si = torch.as_tensor(speech_index, device=dev).to(torch.int64).contiguous()
+        ni = torch.as_tensor(noise_index, device=dev).to(torch.int64).contiguous()
+        B = si.numel()
+        assert ni.numel() == B and B > 0
+        off = None if noise_offset is None else torch.as_tensor(noise_offset, device=dev).to(torch.int32).contiguous()
+        snr = None if snr_db is None else torch.as_tensor(snr_db, device=dev).to(torch.float32).contiguous()
+        assert off is None or off.numel() == B
+        assert snr is None or snr.numel() == B
+        L = self.samples_per_slice * int(n_video_slices)
+        n = min(int(n_video_slices), self.n_frames(L) // self.spss)
+        res = {} if out is None else out
+
+        def buf(name, shape, dtype):
+            t = res.get(name)
+            if t is None or tuple(t.shape) != tuple(shape) or t.dtype != dtype:
+                t = res[name] = torch.empty(shape, dtype=dtype, device=dev)
+            return t
+
+        shape = (B, n, self.n_mels, self.spss)
+        mixed, speech, noise = (buf(k, shape, torch.float32) for k in ("mixed", "speech", "noise"))
+        pcm = buf("mixed_pcm", (B, L), torch.float32)
+        factor = buf("factor", (B,), torch.float32)
+        keys = res.get("keys")
+        if not isinstance(keys, DbKeys) or keys.max.shape[0] != B:
+            keys = res["keys"] = DbKeys(B, dev)
+        keys.equalizer = keys._eq_buf
+        bad = buf("bad_row_flag", (1,), torch.int32)
+        bad.zero_()
+        a = PoolMixArgs()
+        a.speech_pool, a.speech_len, a.speech_stride, a.n_speech = _ptr(sp), _ptr(slen), _rs(sp), sp.shape[0]
+        a.noise_pool, a.noise_len, a.noise_stride, a.n_noise = _ptr(nz), _ptr(nlen), _rs(nz), nz.shape[0]
+        a.sample_format = SAMPLE_I16 if i16 else SAMPLE_F32
+        a.speech_index, a.noise_index, a.noise_offset, a.snr_db = _ptr(si), _ptr(ni), _ptr(off), _ptr(snr)
+        a.B, a.L, a.n_slices = B, L, n
+        a.out_speech, a.out_noise, a.out_mixed, a.out_stride = _ptr(speech), _ptr(noise), _ptr(mixed), _rs(mixed)
+        a.mixed_pcm, a.pcm_stride = _ptr(pcm), _rs(pcm)
+        a.factor_out, a.equalizer_out = _ptr(factor), _ptr(keys.equalizer)
+        a.max_key, a.min_key, a.bad_row_flag = _ptr(keys.max), _ptr(keys.min), _ptr(bad)
+        _native.check(self._lib.avse_mix_pooled(self._ctx, ctypes.byref(a), self._stream()), "avse_mix_pooled")   # (`check` is the flag here)
+        if info is not None:
+            ok = (si >= 0) & (si < sp.shape[0]) & (ni >= 0) & (ni < nz.shape[0])
+            ln = nlen[ni.clamp(0, nz.shape[0] - 1)].clamp(0, _rs(nz))
+            o = torch.zeros_like(ln) if off is None else off
+            ok &= (o >= 0) & (o < ln)
+            info["factor"], info["keys"], info["valid"] = factor, keys, ok & torch.isfinite(factor)
+        if check and int(bad.item()):
+            raise IndexError("mix_pools: a row has an index outside its pool or a noise offset outside [0, noise length)")
+        return mixed, speech, noise, pcm
 
     @_on_device
     def spectrogram(self, signals, lengths=None, stft=False):
@@ -696,6 +768,114 @@ class CorpusDriver(object):
         if self.rank != dst:
             return None
         return torch.cat([p[:k] for p, k in zip(pieces, sizes)])
+
+
+def pack_clips(clips, device=None, dtype=torch.float32, allow_empty=True):
+    """A list of 1-D clips (numpy arrays, tensors or AudioSignal objects) -> (pool [N, stride], lengths [N] int32) on `device`,
+    the layout SpectralEngine.mix_pools and DynamicMixer read: clip k in row k, zeros after its length, stride = the longest
+    clip rounded up to a multiple of 4 samples (aligned vector loads).  dtype torch.int16 keeps raw WAV samples (decoded in
+    the kernels).  allow_empty=False rejects an empty clip -- pack noise pools that way: a row that draws an empty noise clip
+    is invalid (there is nothing to tile, dp:125-126)."""
+    datas = [np.asarray(c.get_data() if hasattr(c, "get_data") else (c.cpu().numpy() if torch.is_tensor(c) else c)) for c in clips]
+    if not datas:
+        raise ValueError("pack_clips: no clips")
+    for k, d in enumerate(datas):
+        if d.ndim != 1:
+            raise ValueError("pack_clips: clip %d is not 1-D (shape %s)" % (k, d.shape))
+        if not allow_empty and d.size == 0:
+            raise ValueError("pack_clips: clip %d is empty" % k)
+    lengths = np.array([d.size for d in datas], dtype=np.int64)
+    if lengths.max() > 0x7fffffff:
+        raise ValueError("pack_clips: clips longer than 2^31 - 1 samples")
+    stride = max(4, (int(lengths.max()) + 3) // 4 * 4)
+    np_dtype = np.int16 if dtype == torch.int16 else np.float32
+    host = np.zeros((len(datas), stride), dtype=np_dtype)
+    for k, d in enumerate(datas):
+        host[k, :d.size] = d
+    return torch.from_numpy(host).to(device), torch.from_numpy(lengths.astype(np.int32)).to(device)
+
+
+def draw_pairings(generator, B, n_speech, noise_lengths, snr_db=(-10.0, 10.0)):
+    """The random pairing of one DynamicMixer epoch, drawn on the host from `generator` (a CPU torch.Generator: the same seed
+    gives the same pairing on any machine).  Returns CPU tensors (speech_index int64, noise_index int64, noise_offset int32,
+    snr_db float32), each [B]:
+      speech_index -- a fresh permutation of range(n_speech), repeated and cut to B: every clip appears floor(B / n_speech)
+                      or ceil(B / n_speech) times;
+      noise_index  -- uniform over the noise pool (noise_lengths [Nn], all > 0);
+      noise_offset -- uniform in [0, Ln) of the drawn noise clip;
+      snr_db       -- uniform in [lo, hi) for a (lo, hi) tuple, a uniform choice among the values of a list, or a constant."""
+    B, n_speech = int(B), int(n_speech)
+    nl = torch.as_tensor(noise_lengths).to("cpu", torch.int64)
+    if B <= 0 or n_speech <= 0 or nl.numel() == 0:
+        raise ValueError("draw_pairings: need B > 0 and non-empty pools")
+    if bool((nl <= 0).any()):
+        raise ValueError("draw_pairings: empty noise clip in the pool")
+    perm = torch.randperm(n_speech, generator=generator)
+    speech_index = perm.repeat((B + n_speech - 1) // n_speech)[:B].contiguous()
+    noise_index = torch.randint(0, nl.numel(), (B,), generator=generator, dtype=torch.int64)
+    ln = nl[noise_index]
+    u = torch.rand(B, generator=generator, dtype=torch.float64)
+    noise_offset = torch.minimum((u * ln.to(torch.float64)).to(torch.int64), ln - 1).to(torch.int32)
+    if isinstance(snr_db, tuple):
+        lo, hi = float(snr_db[0]), float(snr_db[1])
+        snr = (lo + (hi - lo) * torch.rand(B, generator=generator, dtype=torch.float64)).to(torch.float32)
+    elif isinstance(snr_db, (list, np.ndarray)) or torch.is_tensor(snr_db):
+        values = torch.as_tensor(np.asarray(snr_db, dtype=np.float32).reshape(-1))
+        snr = values[torch.randint(0, values.numel(), (B,), generator=generator, dtype=torch.int64)]
+    else:
+        snr = torch.full((B,), float(snr_db), dtype=torch.float32)
+    return speech_index, noise_index, noise_offset, snr.contiguous()
+
+
+class DynamicMixer(object):
+    """Fresh (speech, noise, noise offset, SNR) combinations every training epoch, mixed on the device from two clip pools
+    without materialising any pairing (SpectralEngine.mix_pools).  The reference mixes each speech file with one noise file
+    once, at 0 dB from noise sample 0, and re-reads those frozen mixtures every epoch (speech_enhancer.py:17-58).
+
+    All clips of a mixer share one n_video_slices (L = samples_per_slice * n_video_slices): a corpus with several
+    durations builds one mixer per duration, as preprocess_data buckets.  Pairings come from the mixer's own torch.Generator
+    (seeded with `seed`): the same seed and the same sequence of calls give bit-identical epochs.  In a multi-GPU job give
+    every rank its own seed.
+
+    One epoch, chained into make_sample_set (video rows are indexed by speech_index, like the reference's sample list)::
+
+        speech_pool, speech_len = pack_clips(speech_clips, eng.device)
+        noise_pool, noise_len = pack_clips(noise_clips, eng.device, allow_empty=False)
+        mixer = DynamicMixer(eng, speech_pool, speech_len, noise_pool, noise_len, n_video_slices=15, snr_db=(-10.0, 10.0), seed=rank)
+        for epoch in range(n_epochs):
+            pairing = mixer.draw(3 * len(speech_clips))            # three noisy versions of every clip per epoch
+            mixed, speech, noise, pcm, valid = mixer.mix(pairing)
+            n = torch.where(valid, clip_slices[pairing[0]], 0)     # clip_slices: min(video, audio) slices per speech clip
+            X_mixed, X_speech, perm = eng.make_sample_set(mixed, speech, n_slices=n)
+    """
+
+    def __init__(self, engine, speech_pool, speech_lengths, noise_pool, noise_lengths, n_video_slices, snr_db=(-10.0, 10.0), seed=0):
+        self.eng = engine
+        self.device = engine.device
+        self.speech_pool, self.noise_pool = speech_pool, noise_pool
+        self.speech_lengths = torch.as_tensor(speech_lengths).to(self.device, torch.int32)
+        self.noise_lengths = torch.as_tensor(noise_lengths).to(self.device, torch.int32)
+        self._noise_lengths_host = self.noise_lengths.cpu()           # the offset draw needs them on the host (one copy, here)
+        if bool((self._noise_lengths_host <= 0).any()):
+            raise ValueError("DynamicMixer: the noise pool holds an empty clip (pack it with pack_clips(..., allow_empty=False))")
+        self.n_video_slices = int(n_video_slices)
+        self.snr_db = snr_db
+        self.generator = torch.Generator()
+        self.generator.manual_seed(int(seed))
+
+    def draw(self, B):
+        """(speech_index, noise_index, noise_offset, snr_db) device tensors of B fresh rows (see draw_pairings)."""
+        pairing = draw_pairings(self.generator, B, self.speech_pool.shape[0], self._noise_lengths_host, self.snr_db)
+        return tuple(t.to(self.device) for t in pairing)
+
+    def mix(self, pairing, out=None):
+        """mix_pools of a drawn pairing: (mixed, speech, noise, mixed_pcm, valid), valid [B] bool = factor finite (a silent noise
+        window gives inf / nan).  Asynchronous: nothing is read back."""
+        info = {}
+        si, ni, off, snr = pairing
+        mixed, speech, noise, pcm = self.eng.mix_pools(self.speech_pool, self.speech_lengths, self.noise_pool, self.noise_lengths, si, ni,
+                                                       self.n_video_slices, noise_offset=off, snr_db=snr, out=out, info=info, check=False)
+        return mixed, speech, noise, pcm, info["valid"]
 
 
 def fit_noise(noise, n_noise, n_speech_max):

@@ -134,6 +134,53 @@ int avse_floor_inplace(avse_ctx* ctx, float* data, long long stride, long long n
 int avse_floor_inplace3(avse_ctx* ctx, float* speech, float* noise, float* mixed, long long stride, long long n_per_utt,
                         int B, const int* max_key, const int* min_key, void* stream);
 
+/* Dynamic mixing for training: preprocess_audio_pair (dp:119-139) of pairings drawn from two device-resident clip pools,
+ * without materialising them.  Output row b < B mixes s = the first Ls = speech_len[speech_index[b]] samples of that speech
+ * clip with the noise n[i] = z[(off + i) mod Ln], i < Ls, where z = the first Ln = noise_len[noise_index[b]] samples of that
+ * noise clip and off = noise_offset[b]: off = 0 is the reference's own rule (tile a short noise, dp:125-126, truncate a long
+ * one, dp:128).  factor = sqrt(var(s) / var(n)) * 10^(-snr_db[b]/20) over the Ls samples (dp:130, float64 sums); the speech
+ * always starts at its sample 0 (its video slices are aligned to it, dp:164) and is zero padded / truncated to L (dp:36-42).
+ * A row is INVALID when an index is out of range or off is outside [0, Ln) (so every empty noise clip): it reads no sample,
+ * is processed as an empty pair (factor 0, every slice at the amin floor -100 dB, PCM zeros) and sets *bad_row_flag.
+ * A silent noise window gives inf / nan like numpy (avse_snr_factor).
+ * Enqueues the statistics pass, the forward pass and avse_floor_inplace3 on `stream`; allocates nothing.  Works on every
+ * context avse_forward serves pair batches on (F4, 2-frame and generic-geometry kernels), float32 or int16 pools under the
+ * same rules as avse_forward. */
+typedef struct avse_pool_mix_args {
+    /* pools */
+    const void* speech_pool;        /* [n_speech][speech_stride], float32 or int16 (sample_format) */
+    const int* speech_len;          /* [n_speech] clip lengths; clamped to [0, speech_stride] */
+    long long speech_stride;        /* elements between consecutive clips */
+    long long n_speech;
+    const void* noise_pool;         /* [n_noise][noise_stride], same sample format */
+    const int* noise_len;           /* [n_noise]; clamped to [0, noise_stride] */
+    long long noise_stride;
+    long long n_noise;
+    int sample_format;              /* AVSE_SAMPLE_F32 or AVSE_SAMPLE_I16 */
+    /* pairing of each output row b < B */
+    const long long* speech_index;  /* [B] int64 */
+    const long long* noise_index;   /* [B] int64 */
+    const int* noise_offset;        /* [B] int32 phase of the noise, NULL: 0 for every row */
+    const float* snr_db;            /* [B] or NULL: 0 dB */
+    int B;
+    int L;                          /* signal_length = samples_per_slice * n_video_slices (dp:37) */
+    int n_slices;                   /* slices kept per row, 1 <= n_slices <= int(T / 20) (dp:50, dp:164) */
+    /* outputs */
+    float* out_speech;              /* SLICES [B][n_slices][80][20], floored dB (all three required, 16-byte aligned) */
+    float* out_noise;
+    float* out_mixed;
+    long long out_stride;           /* elements between rows, multiple of 4 */
+    float* mixed_pcm;               /* [B][pcm_stride] s + factor * n zero padded / truncated to L, or NULL */
+    long long pcm_stride;
+    float* factor_out;              /* [B] SNR factor, required */
+    float* equalizer_out;           /* [B] sqrt(var_s / var_n), or NULL (see avse_forward_args::equalizer) */
+    int* max_key;                   /* [B][3] caller scratch (running dB maxima), required */
+    int* min_key;                   /* [B][3] caller scratch (running minima: lets the floor skip rows), or NULL */
+    int* bad_row_flag;              /* device int the caller zeroed; set to 1 when any row is invalid; required */
+} avse_pool_mix_args;
+
+int avse_mix_pooled(avse_ctx* ctx, const avse_pool_mix_args* args, void* stream);
+
 /* dp:49-57 segment gather with the floor applied: SPEC [B][80][ld_t] -> SLICES [B][n_slices][80][20]. */
 int avse_floor_gather(avse_ctx* ctx, const float* spec, long long spec_stride, int ld_t,
                       float* slices, long long slices_stride, int n_slices, int B,
