@@ -170,6 +170,21 @@ bool build_tables(HostTables& t, int sample_rate, double fmin, double fmax) {
         t.tri_ipiv[i] = (float)(1.0 / piv[i]);
         t.tri_sup[i] = (float)sup[i];
     }
+    {   // 1-norm condition number ||G||_1 ||G^-1||_1, the columns of G^-1 by the float64 Thomas factors
+        double g_norm = 0.0, ginv_norm = 0.0;
+        std::vector<double> x(NMEL);
+        for (int j = 0; j < NMEL; ++j) {
+            g_norm = std::max(g_norm, std::fabs(sub[j]) + diag[j] + std::fabs(sup[j]));
+            for (int i = 0; i < NMEL; ++i) x[i] = i == j ? 1.0 : 0.0;
+            for (int i = 1; i < NMEL; ++i) x[i] -= sub[i] / piv[i - 1] * x[i - 1];
+            x[NMEL - 1] /= piv[NMEL - 1];
+            for (int i = NMEL - 2; i >= 0; --i) x[i] = (x[i] - sup[i] * x[i + 1]) / piv[i];
+            double s = 0.0;
+            for (int i = 0; i < NMEL; ++i) s += std::fabs(x[i]);
+            ginv_norm = std::max(ginv_norm, s);
+        }
+        t.gram_cond = g_norm * ginv_norm;
+    }
 
     // ---- SPIKE partition of the same system (see avse_tables.h): everything in float64, rounded once ----
     {
@@ -329,6 +344,11 @@ bool build_tables(HostTables& t, int sample_rate, double fmin, double fmax) {
             if (n4[m] == 1) t.scan4_loc[m * 4 + 1] = ZERO4 | ((ZERO4 + 2) << 16);
         }
     }
+
+    // The I8 inverse is the only inverse of a specialised context: it needs the walk tables, and its float32 solve of
+    // F F^T x = y drifts from pinv (dp:112) in proportion to cond(F F^T) (GRAM_COND_MAX).  Refused banks go to the generic kernels.
+    if (!t.post_ok) { t.error = "filterbank columns do not form a walk (unsupported by the I8 inverse post stage)"; return false; }
+    if (!(t.gram_cond <= GRAM_COND_MAX)) { t.error = "F F^T too ill-conditioned for the float32 tridiagonal solve"; return false; }
     return true;
 }
 

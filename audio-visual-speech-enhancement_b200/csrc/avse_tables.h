@@ -14,6 +14,10 @@ constexpr int SPIKE_P = 4;            // partitions of the 80-band tridiagonal s
 constexpr int SPIKE_Q = NMEL / SPIKE_P;   // 20 bands each
 constexpr int SPIKE_ROW = 5 * SPIKE_Q + 16;   // 116 floats per partition
 static_assert(SPIKE_P * SPIKE_Q == NMEL, "partition of the mel bands");
+// Largest 1-norm cond(F F^T) build_tables accepts.  The I8 inverse's float32 solve drifts from np.linalg.pinv (dp:112) by about
+// 1.5e-11 * cond of the output's peak (emulated I8 kernel, 16 kHz sweep of fmin 0...1500 / fmax 2000...8000): at cond <= 1e5 the
+// error stays <= 1e-5, 10x under the 1e-4 gate; the first bank over the gate is at cond 5.6e6, 56x above this threshold.
+constexpr double GRAM_COND_MAX = 1e5;
 
 struct HostTables {
     int sample_rate = 16000;
@@ -44,6 +48,7 @@ struct HostTables {
     std::vector<float> tri_w;         // [80] Thomas forward multipliers (w[0] unused)
     std::vector<float> tri_ipiv;      // [80] 1 / pivot
     std::vector<float> tri_sup;       // [80] super-diagonal (sup[79] unused)
+    double gram_cond = 0.0;           // 1-norm condition number of F F^T (float64)
     // the same solve partitioned for a warp (I8 inverse kernel): 4 blocks of 20 bands, "SPIKE" form -- per block the local Thomas
     // factors (w, 1/pivot, super-diagonal), the left / right spikes A_p^-1 (T[r0][r0-1] e_0), A_p^-1 (T[r0+19][r0+20] e_19) and the
     // two rows of the inverse 8 x 8 interface system that give x[r0-1] and x[r0+20] from the blocks' local (top, bottom) values
@@ -52,7 +57,8 @@ struct HostTables {
     std::vector<float> col_w;         // [321][2] their weights (0 when absent)
     // the same columns as a walk (I8 post stage): bin k reads the coefficient pair (y[post_b[k]], y[post_b[k] + 1]) with weights
     // post_w[k]; post_b is non-decreasing in steps of <= 1 and stays in [0, 78], so a lane walking a chunk of bins keeps the pair
-    // in registers and advances it on the bits of a mask.  post_ok == false: the filterbank does not allow it (I4 kernel serves).
+    // in registers and advances it on the bits of a mask.  post_ok == false: the filterbank does not allow it; build_tables then
+    // refuses the bank (the I8 kernel is the specialised context's only inverse) and the generic kernels serve it.
     bool post_ok = false;
     std::vector<int> post_b;          // [328]
     std::vector<float> post_w;        // [328][2]
@@ -63,7 +69,8 @@ struct HostTables {
 
 // Fills all tables.  Returns false (and sets t.error) when the configuration cannot be
 // represented in banded form (empty band, band wider than MEL_WMAX, column with > 2 non-zeros,
-// F F^T not tridiagonal).
+// F F^T not tridiagonal), or when the I8 inverse cannot serve it (post_ok == false, or
+// gram_cond > GRAM_COND_MAX).  The flags and gram_cond are set before the last two checks.
 bool build_tables(HostTables& t, int sample_rate, double fmin, double fmax);
 
 }  // namespace avse

@@ -46,7 +46,12 @@ typedef struct avse_ctx avse_ctx;
 
 /* Builds the constant tables (periodic Hann, FFT twiddles, librosa.filters.mel(sr, 640, 80,
  * fmin, fmax) in banded form, tridiagonal factors of F F^T) in float64 on the host and uploads
- * them to `device`.  Replaces the per-call rebuilds at dp:83-89, dp:104-112. */
+ * them to `device`.  Replaces the per-call rebuilds at dp:83-89, dp:104-112.
+ * Returns AVSE_E_CONFIG for a bank the specialised kernels cannot serve: an empty or non-contiguous band, a band wider than
+ * the banded tables hold, a band touching the DC or Nyquist bin, a filterbank column with more than two taps or whose taps
+ * are not adjacent bands (the inverse's walk tables; e.g. 80 / 3000 Hz or 980 / 6200 Hz at 16 kHz, 50 / 8000 Hz at 24 kHz),
+ * or a 1-norm cond(F F^T) above 1e5 (the float32 tridiagonal solve would drift from pinv(F); e.g. 550 / 4600 Hz at
+ * 16 kHz).  avse_create_ex serves every such bank with the generic kernels. */
 int avse_create(int sample_rate, double fmin, double fmax, int device, avse_ctx** out);
 
 /* Any geometry the reference derives from (sample rate, video frame rate, slice duration): n_fft = int(sr / fps) (dp:44),

@@ -211,23 +211,25 @@ def istft(M, hop_length):
 # ----------------------------------------------------------------------------
 
 
-def signal_to_spectrogram(audio_signal, n_fft, hop_length, mel=True, db=True):  # dp:77-96
+def signal_to_spectrogram(audio_signal, n_fft, hop_length, mel=True, db=True, fmin=0.0, fmax=8000.0):  # dp:77-96
+    """fmin / fmax: the filterbank's band edges (the reference hard-codes 0 / 8000)."""
     signal = audio_signal.get_data(channel_index=0)
     D = stft(signal, n_fft=n_fft, hop_length=hop_length)
     magnitude, phase = magphase(D)
     if mel:
-        fb = mel_filterbank(audio_signal.get_sample_rate(), n_fft, n_mels=80, fmin=0, fmax=8000)
+        fb = mel_filterbank(audio_signal.get_sample_rate(), n_fft, n_mels=80, fmin=fmin, fmax=fmax)
         magnitude = np.dot(fb, magnitude)
     if db:
         magnitude = amplitude_to_db(magnitude)
     return magnitude, phase
 
 
-def reconstruct_signal_from_spectrogram(magnitude, phase, sample_rate, n_fft, hop_length, mel=True, db=True):  # dp:99-116
+def reconstruct_signal_from_spectrogram(magnitude, phase, sample_rate, n_fft, hop_length, mel=True, db=True, fmin=0.0,
+                                        fmax=8000.0):  # dp:99-116
     if db:
         magnitude = db_to_amplitude(magnitude)
     if mel:
-        fb = mel_filterbank(sample_rate, n_fft, n_mels=80, fmin=0, fmax=8000)
+        fb = mel_filterbank(sample_rate, n_fft, n_mels=80, fmin=fmin, fmax=fmax)
         magnitude = np.dot(np.linalg.pinv(fb), magnitude)
     signal = istft(magnitude * phase, hop_length=hop_length)
     return AudioSignal(signal, sample_rate)

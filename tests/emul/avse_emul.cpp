@@ -31,6 +31,29 @@ extern "C" int emul_tables_info(int sample_rate, double fmin, double fmax, int* 
     return 0;
 }
 
+// build_tables' verdict (0 accepted, -2 refused) and out = (scan4_ok, scan_ok, post_ok); cond (may be NULL) = gram_cond.
+// The flags and cond are those computed before the verdict; they are meaningful for a bank refused for post_ok or conditioning.
+extern "C" int emul_table_flags(int sample_rate, double fmin, double fmax, int* out, double* cond) {
+    HostTables h;
+    const bool ok = build_tables(h, sample_rate, fmin, fmax);
+    out[0] = h.scan4_ok; out[1] = h.scan_ok; out[2] = h.post_ok;
+    if (cond) *cond = h.gram_cond;
+    return ok ? 0 : -2;
+}
+
+// The inverse tables of an accepted bank: post_w [328][2], post_mask [8][4], tri (w, 1/pivot, sup) [3][80], spike [4][SPIKE_ROW].
+extern "C" int emul_inverse_tables(int sample_rate, double fmin, double fmax, float* post_w, unsigned* post_mask, float* tri, float* spike) {
+    HostTables h;
+    if (!build_tables(h, sample_rate, fmin, fmax)) return -2;
+    memcpy(post_w, h.post_w.data(), sizeof(float) * h.post_w.size());
+    memcpy(post_mask, h.post_mask.data(), sizeof(unsigned) * h.post_mask.size());
+    memcpy(tri, h.tri_w.data(), sizeof(float) * NMEL);
+    memcpy(tri + NMEL, h.tri_ipiv.data(), sizeof(float) * NMEL);
+    memcpy(tri + 2 * NMEL, h.tri_sup.data(), sizeof(float) * NMEL);
+    memcpy(spike, h.spike.data(), sizeof(float) * h.spike.size());
+    return 0;
+}
+
 // One emulated warp: its private shared-memory region plus the per-lane registers that live across
 // a __syncwarp() in the kernel.
 struct EmulWarp {

@@ -174,3 +174,24 @@ def test_snr_factor_is_invariant_to_the_variance_convention():
         assert abs(f - np.sqrt(np.var(s, ddof=ddof) / np.var(n, ddof=ddof)) * 10 ** (-5.0 / 20)) < 1e-12 * f
     # the mixture then has the requested SNR by construction: 10 log10(var(s) / var(f n)) == snr_db
     assert abs(10 * np.log10(np.var(s) / np.var(f * n)) - 5.0) < 1e-9
+
+
+def test_band_edge_keywords_of_the_spectrogram_functions():
+    """fmin / fmax default to the reference's 0 / 8000 (bit-identical), and otherwise select O.mel_filterbank(sr, n_fft, 80, fmin,
+    fmax) in both directions: amplitude_to_db(fb |stft|) forward, istft((pinv(fb) 10^(mel/20)) phase) back."""
+    x = _sig(8000, 5)
+    sig = O.AudioSignal(x, SR)
+    mag, phase = O.signal_to_spectrogram(sig, NFFT, HOP)
+    mag0, phase0 = O.signal_to_spectrogram(sig, NFFT, HOP, fmin=0.0, fmax=8000.0)
+    assert np.array_equal(mag, mag0) and np.array_equal(phase, phase0)
+    back = O.reconstruct_signal_from_spectrogram(mag, phase, SR, NFFT, HOP).get_data()
+    assert np.array_equal(back, O.reconstruct_signal_from_spectrogram(mag, phase, SR, NFFT, HOP, fmin=0.0, fmax=8000.0).get_data())
+    fb = O.mel_filterbank(SR, NFFT, 80, 300.0, 3500.0)
+    D = O.stft(x, NFFT, HOP)
+    mag2, phase2 = O.signal_to_spectrogram(sig, NFFT, HOP, fmin=300.0, fmax=3500.0)
+    assert np.array_equal(phase2, phase)
+    assert np.max(np.abs(mag2 - O.amplitude_to_db(fb @ np.abs(D)))) < 1e-12
+    assert np.max(np.abs(mag2 - mag)) > 1.0
+    want = O.istft((np.linalg.pinv(fb) @ O.db_to_amplitude(mag2)) * phase2, HOP)
+    got = O.reconstruct_signal_from_spectrogram(mag2, phase2, SR, NFFT, HOP, fmin=300.0, fmax=3500.0).get_data()
+    assert np.max(np.abs(got - want)) < 1e-12 * np.max(np.abs(want))
