@@ -5,6 +5,8 @@
 // 321 bins, 80 Slaney mel bands, 200 ms slices = 20 spectrogram frames.
 #pragma once
 
+#include <cmath>
+
 #if defined(__CUDACC__)
 #define AVSE_HD __host__ __device__ __forceinline__
 #define AVSE_HD_COLD __host__ __device__ __noinline__     // cold helpers: ONE copy, kept out of the hot instruction stream
@@ -154,6 +156,28 @@ AVSE_HD int noise_weight(const NoiseSpan& w, int j, int Ln, int off) {    // per
     int d = j - off;
     d += d < 0 ? Ln : 0;
     return w.q + (d < w.rem ? 1 : 0);
+}
+
+// The statistics pass's epilogue: from the float64 sums t = (sum s, sum s^2, sum n, sum n^2) over the n samples of a pair, the
+// SNR factor f = sqrt(var_s / var_n) 10^(-snr/20) (dp:130, population variances) and the level equaliser g = sqrt(sum s^2 /
+// sum n^2).  The forward kernels pack z = s + i g n into one complex FFT and apply f / g after it, so any g gives s + f n; g only
+// conditions the float32 arithmetic.  Rounding of either channel leaks into the other in proportion to its RAW power, mean
+// included (a DC offset goes through the window and the FFT like any other component), so g balances the raw powers, not the
+// variances.  n == 0 (empty files) gives f = g = 0; a silent noise gives inf / nan for both, like numpy; a constant non-zero
+// noise (var_n == 0) gives a finite g and a non-finite f.
+struct SnrGains { float factor, equalizer; };
+AVSE_HD SnrGains snr_gains(int n, const double (&t)[4], double snr_db) {
+    SnrGains r;
+    r.factor = 0.0f;
+    r.equalizer = 0.0f;
+    if (n > 0) {
+        const double inv = 1.0 / (double)n;
+        const double ms = t[0] * inv, mn = t[2] * inv;
+        const double vs = t[1] * inv - ms * ms, vn = t[3] * inv - mn * mn;
+        r.factor = (float)(sqrt(vs / vn) * pow(10.0, -snr_db / 20.0));
+        r.equalizer = (float)sqrt(t[1] / t[3]);
+    }
+    return r;
 }
 
 #if defined(__CUDACC__)

@@ -95,10 +95,10 @@ struct FwdTileT {
     int T;               // STFT frames: 1 + L / hop
     int t0;              // first frame of the group (multiple of FPG)
     // The SNR factor f (dp:130) is applied in two parts, f = gain * factor: the noise is multiplied by `gain`
-    // (= sqrt(var_s / var_n), the level equaliser) as it is LOADED, so that the two channels of the packed FFT
-    // z = s + i (gain n) carry equal power whatever the raw levels of the two files (float vs int16 scale ...):
-    // fp32 rounding of the louder channel would otherwise leak into the quieter one through the unpack
-    // S' = Z_k + conj Z_{N-k}.  The residual `factor` (= 10^(-snr/20), exactly 1 at the reference's 0 dB) is applied
+    // (= sqrt(sum s^2 / sum n^2), the level equaliser) as it is LOADED, so that the two channels of the packed FFT
+    // z = s + i (gain n) carry equal raw power whatever the levels and DC offsets of the two files (float vs int16
+    // scale ...): fp32 rounding of the louder channel would otherwise leak into the quieter one through the unpack
+    // S' = Z_k + conj Z_{N-k}.  The residual `factor` = f / gain (10^(-snr/20) for zero-mean files) is applied
     // after the unpack by STFT linearity.
     float gain;          // applied to the noise samples at load; 0 when nz == nullptr
     float factor;        // residual applied to the (gain-scaled) noise spectrum / mel sums; 0 when nz == nullptr

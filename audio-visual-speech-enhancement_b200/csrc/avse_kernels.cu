@@ -311,19 +311,10 @@ __global__ void __launch_bounds__(256) avse_snr_factor_kernel(const S* __restric
             t[0] += qq[0]; t[1] += qq[1]; t[2] += qq[2]; t[3] += qq[3];
         }
         // n == 0 (empty files): the reference mixes two empty arrays and pads with zeros (dp:39-40); nothing is scaled,
-        // so any finite factor gives its result: use 0.  var(noise) == 0 with n > 0 gives inf / nan exactly like numpy.
-        float g = 0.0f, f = 0.0f;
-        if (n > 0) {
-            const double inv = 1.0 / (double)n;
-            const double ms = t[0] * inv, mn = t[2] * inv;
-            const double vs = t[1] * inv - ms * ms, vn = t[3] * inv - mn * mn;
-            const double db = snr_db ? (double)snr_db[u] : 0.0;
-            const double eq = sqrt(vs / vn);
-            g = (float)eq;
-            f = (float)(eq * pow(10.0, -db / 20.0));
-        }
-        factor_out[u] = f;
-        if (equalizer_out) equalizer_out[u] = g;
+        // so any finite factor gives its result: 0.  var(noise) == 0 with n > 0 gives inf / nan exactly like numpy.
+        const SnrGains r = snr_gains(n, t, snr_db ? (double)snr_db[u] : 0.0);
+        factor_out[u] = r.factor;
+        if (equalizer_out) equalizer_out[u] = r.equalizer;
         if (max_key) { max_key[3 * u] = (int)0x80000000; max_key[3 * u + 1] = (int)0x80000000; max_key[3 * u + 2] = (int)0x80000000; }
         if (min_key) { min_key[3 * u] = 0x7fffffff; min_key[3 * u + 1] = 0x7fffffff; min_key[3 * u + 2] = 0x7fffffff; }
     }

@@ -49,8 +49,8 @@ class DbKeys(object):
     """Per-utterance side data that the statistics pass (avse_snr_factor) hands to the forward pass, device resident:
     the running dB extrema of (speech, noise, mixed) as order-preserving int32 keys -- `max` [B, 3] over all frames
     (librosa's top_db reference, dp:94), `min` [B, 3] over the stored values (lets the floor pass skip utterances that
-    need no clipping) -- and `equalizer` [B] = sqrt(var_s / var_n), the level-equalising part of the SNR factor
-    (avse_forward_args::equalizer; None until snr_factor has filled it)."""
+    need no clipping) -- and `equalizer` [B] = sqrt(sum s^2 / sum n^2), the ratio of the raw powers of speech and noise that
+    conditions the packed FFT of the forward kernels (avse_forward_args::equalizer; None until snr_factor has filled it)."""
     __slots__ = ("buf", "max", "min", "equalizer", "_eq_buf")
 
     def __init__(self, B, device):

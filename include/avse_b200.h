@@ -78,8 +78,10 @@ int avse_get_filterbank(const avse_ctx* ctx, double* host_out);
  * noise_period (may be NULL): [B] own length Ln of each noise file.  Where Ln < lengths[u] the noise is the periodic tiling
  *   noise[i] = nz[i mod Ln] -- what the reference's "double until long enough, then truncate" loop builds (dp:125-128) --
  *   and only the first Ln samples of the noise row are read.
- * equalizer_out (may be NULL): [B] sqrt(var(speech_u) / var(noise_u)) alone, the part of the factor that equalises the
- *   levels of the two files; hand it to avse_forward (avse_forward_args::equalizer).
+ * equalizer_out (may be NULL): [B] sqrt(sum s^2 / sum n^2), the ratio of the RAW powers (mean included) of speech and noise
+ *   over exactly the samples the factor uses (the first lengths[u], the weighted period of a tiled noise, the window of a
+ *   pooled row); hand it to avse_forward (avse_forward_args::equalizer).  0 where lengths[u] == 0; finite for a constant
+ *   non-zero noise, whose factor is non-finite.
  * lengths[u] == 0 gives factor 0 (the reference mixes two empty arrays and zero-pads them, dp:39-40); a silent noise
  * (variance 0) gives inf / nan like numpy, and so does everything computed from it.
  * Also resets max_key[u][0..2] (the running dB maxima used by avse_forward / avse_floor_*) and, when
@@ -117,9 +119,10 @@ typedef struct avse_forward_args {
                                 for pair batches (noise != NULL) without stft_speech */
     const float* equalizer;  /* [B] from avse_snr_factor (equalizer_out), or NULL.  Numerical conditioning only: results are the
                                 reference's s + factor * n either way.  The float32 kernels carry speech and noise through ONE
-                                packed complex FFT; with the noise pre-scaled by equalizer[u] = sqrt(var_s / var_n) both channels
-                                have equal power whatever the raw levels of the two files (a float WAV next to an int16 one ...),
-                                and the remaining factor[u] / equalizer[u] = 10^(-snr/20) is applied by STFT linearity.
+                                packed complex FFT, where float32 rounding of each channel leaks into the other in proportion to
+                                its raw power; with the noise pre-scaled by equalizer[u] = sqrt(sum s^2 / sum n^2) both channels
+                                have equal raw power whatever the levels and DC offsets of the two files (a float WAV next to an
+                                int16 one ...), and the remaining factor[u] / equalizer[u] is applied by STFT linearity.
                                 NULL: the whole factor is applied before the transform */
     const int* noise_period; /* [B] or NULL: own length Ln of each noise file; where Ln < len_noise[u] the kernels read
                                 noise[i mod Ln] (dp:125-128) and only the first Ln samples of the noise row need to exist */
@@ -178,7 +181,7 @@ typedef struct avse_pool_mix_args {
     float* mixed_pcm;               /* [B][pcm_stride] s + factor * n zero padded / truncated to L, or NULL */
     long long pcm_stride;
     float* factor_out;              /* [B] SNR factor, required */
-    float* equalizer_out;           /* [B] sqrt(var_s / var_n), or NULL (see avse_forward_args::equalizer) */
+    float* equalizer_out;           /* [B] sqrt(sum s^2 / sum n^2), or NULL (see avse_forward_args::equalizer) */
     int* max_key;                   /* [B][3] caller scratch (running dB maxima), required */
     int* min_key;                   /* [B][3] caller scratch (running minima: lets the floor skip rows), or NULL */
     int* bad_row_flag;              /* device int the caller zeroed; set to 1 when any row is invalid; required */

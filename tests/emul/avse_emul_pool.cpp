@@ -181,3 +181,15 @@ extern "C" int emul_noise_sums(const float* z, int Ln, int n, int off, double* o
     out2[1] = b1;
     return w.periodic ? 1 : 0;
 }
+
+// The whole statistics pass of one pair: speech s[0, n), noise n[i] = z[(off + i) mod Ln] (Ln = n, off = 0 for a plain row),
+// float64 sums in one thread's order, then the kernel's epilogue snr_gains (avse_common.h).  out2 = (factor, equalizer).
+extern "C" int emul_snr_gains(const float* s, int n, const float* z, int Ln, int off, double snr_db, float* out2) {
+    double t[4] = {0.0, 0.0, 0.0, 0.0};
+    for (int i = 0; i < n; ++i) { const double v = s[i]; t[0] += v; t[1] += v * v; }
+    const int periodic = n > 0 ? emul_noise_sums(z, Ln, n, off, t + 2) : 0;
+    const SnrGains r = snr_gains(n, t, snr_db);
+    out2[0] = r.factor;
+    out2[1] = r.equalizer;
+    return periodic;
+}

@@ -253,7 +253,8 @@ def test_f4_stage_code_fuzz_against_oracle(emul):
                snr=st.floats(-10.0, 10.0), seed=st.integers(0, 10 ** 6))
     def check(nvs, frac, log_scale, log_nscale, snr, seed):
         # speech and noise levels are drawn INDEPENDENTLY (a float WAV next to an int16 one ...): the level equaliser
-        # g = sqrt(var_s / var_n) goes to the kernel stages as `gain`, the full factor g 10^(-snr/20) as `factor`
+        # g goes to the kernel stages as `gain`, the full factor as `factor`; zero-mean noise: sqrt(sum s^2 / sum n^2) is
+        # within rounding of the ratio of standard deviations used here
         L = 3200 * nvs
         nv = max(330, min(L, int(frac * L)))
         rng = np.random.RandomState(seed)
@@ -286,7 +287,7 @@ LEVELS = [(1.0, 1.0), (1.0, 10.0), (1.0, 100.0), (1.0, 32767.0), (100.0, 1.0), (
 @pytest.mark.parametrize("snr", [-10.0, 0.0, 10.0])
 def test_level_mismatch_holds_the_gate(emul, snr, f2):
     """dp:130-133 exists precisely for files recorded at different levels.  With the noise equalised to the speech power
-    before the packed FFT (gain = sqrt(var_s / var_n)) and only 10^(-snr/20) applied by linearity, the three log-mels
+    before the packed FFT (gain = sqrt(sum s^2 / sum n^2), the statistics pass's equaliser) and only the rest applied by linearity, the three log-mels
     stay within 1e-3 dB of the float64 oracle and the mixture PCM within 1e-4 of full scale for raw level ratios from
     1e-4 to 3e4 (float WAV vs int16 WAV) at -10 / 0 / +10 dB."""
     L = 16000
