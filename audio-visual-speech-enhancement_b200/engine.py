@@ -77,6 +77,19 @@ def geometry(sample_rate, video_frame_rate, slice_duration_ms=200):
     return samples_per_slice, n_fft, hop, spss
 
 
+def frame_count(L, n_fft, hop):
+    """librosa.stft(center=True) frame count of a length-L signal: 1 + (L + 2 (n_fft // 2) - n_fft) // hop."""
+    return 1 + (int(L) + 2 * (n_fft // 2) - n_fft) // hop
+
+
+def slice_count(L, n_fft, hop, spss):
+    """Slices of a length-L signal, int(T / spss) (dp:50).  This is the count preprocess_audio_pair returns; the
+    min(video, audio) cut of dp:164 comes later, in data_processor.assemble_sample.  It exceeds n_video_slices
+    (L = samples_per_slice * n_video_slices) when spss * hop < samples_per_slice, e.g. from 65 slices on at 16 kHz /
+    24000/1001 fps."""
+    return frame_count(L, n_fft, hop) // spss
+
+
 class SpectralEngine(object):
     """One GPU's worth of the spectral front/back end."""
 
@@ -151,7 +164,11 @@ class SpectralEngine(object):
 
     def n_frames(self, L):
         """librosa.stft(center=True) frame count: 1 + (L + 2 (n_fft // 2) - n_fft) // hop (== 1 + L // hop for even n_fft)."""
-        return 1 + (L + 2 * (self.n_fft // 2) - self.n_fft) // self.hop
+        return frame_count(L, self.n_fft, self.hop)
+
+    def n_slices(self, L):
+        """Slices a length-L row yields, int(T / spss) (dp:50; see slice_count)."""
+        return slice_count(L, self.n_fft, self.hop, self.spss)
 
     # ------------------------------------------------------------------ a3: SNR factor
     @_on_device
@@ -195,7 +212,7 @@ class SpectralEngine(object):
             assert _rs(noise) == _rs(speech) and noise.shape[0] == B
         T = self.n_frames(L)
         if n_slices is None:
-            n_slices = T // self.spss
+            n_slices = self.n_slices(L)
         res = {} if out is None else out
         ld_t = (T + 3) // 4 * 4
         shape = (B, n_slices, self.n_mels, self.spss) if layout == LAYOUT_SLICES else (B, self.n_mels, ld_t)
@@ -289,14 +306,14 @@ class SpectralEngine(object):
         speech, noise: [B, >=max(lengths)] float32 or int16, same row stride.  noise_lengths [B] int32 (optional): own
         length of each noise file -- a noise shorter than its speech is tiled periodically inside the kernels
         (dp:125-128); without it the noise rows must already cover the speech length (see fit_noise).
-        Returns (mixed_slices, speech_slices, noise_slices, mixed_pcm) with shapes [B, n, 80, 20] x3 and [B, L];
-        n = min(n_video_slices, int(T/20)) (dp:50, dp:164).  Batches of any size: nothing here is capped at 65 535.
+        Returns (mixed_slices, speech_slices, noise_slices, mixed_pcm) with shapes [B, n, 80, spss] x3 and [B, L];
+        n = int(T / spss) (dp:50, see slice_count), L = samples_per_slice * n_video_slices.  Batches of any size: nothing
+        here is capped at 65 535.
         """
         i16 = speech.dtype == torch.int16 and noise.dtype == torch.int16
         speech, noise = self._as_batch(speech, i16), self._as_batch(noise, i16)
         L = self.samples_per_slice * int(n_video_slices)
-        T = self.n_frames(L)
-        n = min(int(n_video_slices), T // self.spss)
+        n = self.n_slices(L)
         if lengths is None and speech.shape[1] != L:
             lengths = torch.full((speech.shape[0],), speech.shape[1], dtype=torch.int32, device=self.device)
         # info: optional dict that receives the SNR factors and the dB keys
@@ -319,8 +336,8 @@ class SpectralEngine(object):
         speech_index[b] with noise clip noise_index[b] read from sample noise_offset[b] on and wrapped around its length:
         n[i] = z[(off + i) mod Ln] (off = 0, the default, is the reference's tile-or-truncate rule, dp:125-128), at snr_db[b]
         (default 0 dB, dp:130).  No pairing is materialised.
-        Returns (mixed, speech, noise, mixed_pcm) shaped like preprocess_pairs: [B, n, 80, 20] x3 and [B, L],
-        n = min(n_video_slices, int(T/20)).
+        Returns (mixed, speech, noise, mixed_pcm) shaped like preprocess_pairs: [B, n, 80, spss] x3 and [B, L],
+        n = int(T / spss) (dp:50, see slice_count).
         A row with an index out of range or an offset outside [0, Ln) is invalid: it is processed as an empty pair (every slice
         at -100 dB, PCM zeros).  check=True reads the device flag back (one synchronisation) and raises IndexError; check=False
         stays asynchronous.  out: dict whose tensors are re-used from call to call (like preprocess_pairs / HostPipeline).
@@ -341,7 +358,7 @@ class SpectralEngine(object):
         assert off is None or off.numel() == B
         assert snr is None or snr.numel() == B
         L = self.samples_per_slice * int(n_video_slices)
-        n = min(int(n_video_slices), self.n_frames(L) // self.spss)
+        n = self.n_slices(L)
         res = {} if out is None else out
 
         def buf(name, shape, dtype):
@@ -408,13 +425,12 @@ class SpectralEngine(object):
 
     @_on_device
     def preprocess_signals(self, signals, n_video_slices, lengths=None):
-        """Batched preprocess_audio_signal (dp:35-57): [B, n, 80, 20] floored dB slices."""
+        """Batched preprocess_audio_signal (dp:35-57): [B, n, 80, spss] floored dB slices, n = int(T / spss) (dp:50)."""
         signals = self._as_batch(signals)
         L = self.samples_per_slice * int(n_video_slices)
         if lengths is None and signals.shape[1] < L:
             lengths = torch.full((signals.shape[0],), signals.shape[1], dtype=torch.int32, device=self.device)
-        T = self.n_frames(L)
-        n = T // self.spss
+        n = self.n_slices(L)
         res = self.forward_raw(signals, None, L=L, len_speech=lengths, layout=LAYOUT_SLICES, n_slices=n, want=("speech",), mixed_pcm=False)
         return self.floor_(res["speech"], res["max_key"], 0)
 
@@ -637,7 +653,7 @@ class HostPipeline(object):
         self.eng = engine
         self.L = int(L)
         self.n_video_slices = int(n_video_slices)
-        self.n_slices = min(self.n_video_slices, engine.n_frames(self.L) // engine.spss)
+        self.n_slices = engine.n_slices(self.L)
         self.chunk = int(chunk)
         dev = engine.device
         self.streams = [torch.cuda.Stream(device=dev) for _ in range(n_streams)]

@@ -11,6 +11,7 @@ import pytest
 import torch
 
 from oracle import avse_oracle as O
+from tests.cases import FRAME_RATES, frame_rate_fps
 
 pytestmark = pytest.mark.gpu
 
@@ -18,8 +19,10 @@ TOL_DB = 1e-3
 TOL_PCM = 1e-4
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-# (sample rate, fps): n_fft 320 (16x20), 666 (18x37), 533 (13x41, odd), 1764 (42x42), 320 @ 8 kHz, 1920 (40x48)
-CONFIGS = [(16000, 50.0), (16000, 24.0), (16000, 30.0), (44100, 25.0), (8000, 25.0), (48000, 25.0)]
+# (sample rate, fps): n_fft 320 (16x20), 666 (18x37), 533 (13x41, odd), 1764 (42x42), 320 @ 8 kHz, 1920 (40x48), then the
+# frame rates real videos carry (tests.cases.FRAME_RATES: prime, odd, rank-deficient and the largest sizes)
+CONFIGS = [(16000, 50.0), (16000, 24.0), (16000, 30.0), (44100, 25.0), (8000, 25.0), (48000, 25.0)] + \
+    [(g["sr"], frame_rate_fps(g)) for g in FRAME_RATES]
 
 
 @pytest.fixture(scope="module")

@@ -12,7 +12,7 @@ import pytest
 import torch
 
 from oracle import avse_oracle as O
-from tests.cases import SR, FPS
+from tests.cases import SR, FPS, FRAME_RATES, frame_rate_fps
 
 pytestmark = pytest.mark.gpu
 
@@ -235,7 +235,8 @@ def test_scale_70k_rows_from_small_pools(eng):
     _check_rows([t[rows] for t in out], sp, nz, si[rows], ni[rows], off[rows], snr[rows], nvs, range(len(rows)))
 
 
-OTHER_CONTEXTS = [("f2", 16000, 25.0), ("n320", 16000, 50.0), ("n533", 16000, 30.0), ("n1764", 44100, 25.0)]
+OTHER_CONTEXTS = [("f2", 16000, 25.0), ("n320", 16000, 50.0), ("n533", 16000, 30.0), ("n1764", 44100, 25.0)] + \
+    [(g["name"], g["sr"], frame_rate_fps(g)) for g in FRAME_RATES]
 
 
 @pytest.mark.parametrize("name,sr,fps", OTHER_CONTEXTS, ids=[c[0] for c in OTHER_CONTEXTS])
@@ -261,6 +262,7 @@ def test_other_contexts_match_oracle(mod, name, sr, fps):
     rng = np.random.RandomState(29)
     B, nvs = 8, 6
     si, ni, off, snr = _pairing(rng, B, nl_, len(sp))
+    off[6] = 1                       # rows 0-5 pin offsets 0, Ln - 1 and Ln // 2
     out = e.mix_pools(spP, sl, nzP, nl, _d(si), _d(ni), nvs, noise_offset=_d(off), snr_db=_d(snr))
     torch.cuda.synchronize()
     _check_rows(out, sp, nz, si, ni, off, snr, nvs, range(B), sr, fps)
