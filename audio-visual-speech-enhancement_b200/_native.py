@@ -63,7 +63,7 @@ EXPORTS = [
     "avse_snr_factor", "avse_forward", "avse_floor_inplace", "avse_floor_gather", "avse_reset_max", "avse_max_db",
     "avse_inverse", "avse_inverse_work_elems", "avse_floor_inplace3", "avse_gather_rows",
     "avse_create_ex", "avse_get_geometry", "avse_inverse_work_elems_ctx",
-    "avse_video_stats", "avse_video_normalize", "avse_mse", "avse_magphase", "avse_mix_pooled",
+    "avse_video_stats", "avse_video_normalize", "avse_mse", "avse_magphase", "avse_mix_pooled", "avse_inverse_backward",
 ]
 
 
@@ -105,6 +105,8 @@ def load(build=True):
     lib.avse_max_db.restype = i32
     lib.avse_inverse.argtypes = [vp, _c.POINTER(InverseArgs), vp]
     lib.avse_inverse.restype = i32
+    lib.avse_inverse_backward.argtypes = [vp, _c.POINTER(InverseArgs), vp, ll, vp, vp]
+    lib.avse_inverse_backward.restype = i32
     lib.avse_inverse_work_elems.argtypes = [i32, _c.POINTER(ll)]
     lib.avse_inverse_work_elems.restype = i32
     lib.avse_create_ex.argtypes = [i32, i32, i32, i32, i32, f64, f64, i32, _c.POINTER(vp)]

@@ -14,8 +14,8 @@ ROOT = os.path.dirname(PKG_DIR)
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "libavse_b200.so")
 
-SOURCES = ["avse_kernels.cu", "avse_inverse.cu", "avse_generic.cu", "avse_video.cu", "avse_tables.cpp", "avse_generic_tables.cpp"]
-HEADERS = ["avse_common.h", "avse_dft.cuh", "avse_tables.h", "avse_ctx.h", "avse_fwd_stages.cuh", "avse_fwd4_stages.cuh", "avse_inv_stages.cuh", "avse_inv8_stages.cuh", "avse_generic.h",
+SOURCES = ["avse_kernels.cu", "avse_inverse.cu", "avse_inverse_grad.cu", "avse_generic.cu", "avse_video.cu", "avse_tables.cpp", "avse_generic_tables.cpp"]
+HEADERS = ["avse_common.h", "avse_dft.cuh", "avse_tables.h", "avse_ctx.h", "avse_fwd_stages.cuh", "avse_fwd4_stages.cuh", "avse_inv_stages.cuh", "avse_inv8_stages.cuh", "avse_inverse_grad_stages.cuh", "avse_generic.h",
            os.path.join(ROOT, "include", "avse_b200.h")]
 
 NVCC_FLAGS = [

@@ -30,13 +30,16 @@ struct avse_ctx {
     avse::GenericHost gen;
     avse::GenericDev gd;
     void* gbase = nullptr;        // device allocation holding the generic tables
-    size_t gen_fwd_smem_set = 0, gen_inv_smem_set = 0;   // dynamic shared-memory opt-in already requested through this context
+    size_t gen_fwd_smem_set = 0, gen_inv_smem_set = 0, gen_grad_smem_set = 0;   // dynamic shared-memory opt-in already requested through this context
 };
 
 // pool == nullptr: rows of args->speech / args->noise; otherwise avse_mix_pooled's row indirection into them (avse_common.h)
 int avse_generic_forward(avse_ctx* ctx, const avse_forward_args* args, const avse::PoolRows* pool, void* stream);
 int avse_generic_inverse(avse_ctx* ctx, const avse_inverse_args* args, void* stream);
 int avse_generic_frames(const avse::GenericGeo& q, int L);
+// avse_inverse_backward on a generic-geometry context, arguments already validated
+int avse_generic_inverse_backward(avse_ctx* ctx, const avse_inverse_args* args, int T_use, int t_write, const float* grad_pcm,
+                                  long long grad_pcm_stride, float* grad_mel, void* stream);
 
 int avse_fail(int code, const std::string& msg);
 int avse_cuda_fail(cudaError_t e, const char* where);

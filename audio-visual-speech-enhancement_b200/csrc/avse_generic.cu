@@ -310,12 +310,109 @@ __global__ void __launch_bounds__(256) avse_generic_inverse_ola_kernel(const __g
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// inverse backward: one CTA per (frame, utterance) of grad_mel.  dL/d dB_t = ln(10)/20 a_t pinv(F)^T d_t with
+// d_t[k] = (c_k / n_inv) Re(conj(phi_t[k]) rfft_{n_inv}(w_inv e_t)[k]) (avse_inverse_grad_stages.cuh); float64 transforms
+// and accumulation.  Frames t >= T_use get exact zeros.
+// ---------------------------------------------------------------------------------------------
+struct GenGradParams {
+    avse_inverse_args a;
+    GenericGeo geo;
+    GenericDev d;
+    const float* grad;
+    long long grad_stride;
+    float* grad_mel;
+    int T_use;
+    int t_write;
+    int out_len;
+};
+
+__global__ void __launch_bounds__(GEN_THREADS) avse_generic_inverse_grad_kernel(const __grid_constant__ GenGradParams P) {
+    extern __shared__ __align__(16) unsigned char gsm[];
+    const GenericGeo& q = P.geo;
+    const avse_inverse_args& A = P.a;
+    const int N = q.n_fft, Ni = q.n_inv, bins = q.bins, M = q.n_mels, hop = q.hop;
+    const int NX = N > Ni ? N : Ni;
+    double2* X = reinterpret_cast<double2*>(gsm);
+    double2* Y = X + NX;
+    double2* phi = Y + NX;                               // [bins]
+    double* dk = reinterpret_cast<double*>(Y);           // [bins], once Y is free
+    const int u = blockIdx.x / P.t_write, t = blockIdx.x - u * P.t_write;
+    const int tid = threadIdx.x;
+    size_t base, mstride;
+    if (A.layout == AVSE_LAYOUT_SLICES) {
+        const int sl = t / q.spss, tt = t - sl * q.spss;
+        base = (size_t)sl * M * q.spss + tt;
+        mstride = q.spss;
+    } else {
+        base = t;
+        mstride = A.ld_t;
+    }
+    float* gout = P.grad_mel + (size_t)u * A.mel_stride + base;
+    if (t >= P.T_use) {
+        for (int m = tid; m < M; m += GEN_THREADS) gout[(size_t)m * mstride] = 0.0f;
+        return;
+    }
+    // phase of the mixture's STFT frame (magphase, dp:80)
+    int valid = A.len_pcm ? A.len_pcm[u] : A.L;
+    valid = valid < A.L ? valid : A.L;
+    const float* pcm = A.mixed_pcm + (size_t)u * A.pcm_stride;
+    const int mbase = t * hop - N / 2;
+    for (int n = tid; n < N; n += GEN_THREADS) X[n] = make_double2((double)gen_sample(pcm, mbase + n, A.L, valid) * (double)P.d.window[n], 0.0);
+    __syncthreads();
+    gen_dft(X, Y, X, reinterpret_cast<const double2*>(P.d.tw), N, q.n1, q.n2);
+    for (int k = tid; k < bins; k += GEN_THREADS) {
+        const double2 z = X[k];
+        const double r = hypot(z.x, z.y);
+        phi[k] = r > 0.0 ? make_double2(z.x / r, z.y / r) : make_double2(1.0, 0.0);
+    }
+    __syncthreads();
+    // the gradient frame: e = g at offset n_inv / 2 of the untrimmed signal, / window sum-square where > tiny(float32)
+    const float* g = P.grad + (size_t)u * P.grad_stride;
+    for (int n = tid; n < Ni; n += GEN_THREADS) {
+        const int pp = t * hop + n, o = pp - Ni / 2;
+        double e = 0.0;
+        if (o >= 0 && o < P.out_len) {
+            int t_hi = pp / hop;
+            if (t_hi > P.T_use - 1) t_hi = P.T_use - 1;
+            const int t_lo = pp - Ni + 1 <= 0 ? 0 : (pp - Ni + hop) / hop;
+            float wss = 0.0f;                               // as the forward's overlap-add computes it
+            for (int s = t_lo; s <= t_hi; ++s) {
+                const float wn = P.d.window_inv[pp - s * hop];
+                wss = fmaf(wn, wn, wss);
+            }
+            e = wss > 1.17549435e-38f ? (double)g[o] / (double)wss : (double)g[o];
+        }
+        X[n] = make_double2(e * (double)P.d.window_inv[n], 0.0);
+    }
+    __syncthreads();
+    gen_dft(X, Y, X, reinterpret_cast<const double2*>(P.d.tw_inv), Ni, q.i1, q.i2);
+    for (int k = tid; k < bins; k += GEN_THREADS) {
+        const double2 h = X[k], p = phi[k];
+        const bool edge = k == 0 || 2 * k == Ni;            // C2R reads only the real part of DC / Nyquist
+        dk[k] = edge ? p.x * h.x / (double)Ni : 2.0 * (p.x * h.x + p.y * h.y) / (double)Ni;
+    }
+    __syncthreads();
+    // pinv(F)^T d, dB chain rule (db_to_amplitude, dp:101)
+    const float* mel = A.mel_db + (size_t)u * A.mel_stride + base;
+    for (int m = tid; m < M; m += GEN_THREADS) {
+        double acc = 0.0;
+        for (int k = 0; k < bins; ++k) acc = fma((double)P.d.pinv[(size_t)k * M + m], dk[k], acc);
+        const double amp = (double)exp2f(0.16609640474436813f * mel[(size_t)m * mstride]);
+        gout[(size_t)m * mstride] = (float)(0.11512925464970229 * amp * acc);
+    }
+}
+
 constexpr size_t kGenMaxSmem = 227 * 1024;   // opt-in ceiling of sm_100 (n_fft <= 4096 needs <= 157 KB)
 
 size_t gen_fwd_smem(const GenericGeo& q) { return (size_t)q.n_fft * 32 + (size_t)q.bins * 12 + 32; }
 size_t gen_inv_smem(const GenericGeo& q) {
     const size_t nx = q.n_fft > q.n_inv ? q.n_fft : q.n_inv;
     return nx * 32 + (size_t)(q.n_mels + q.bins) * 4 + 16;
+}
+size_t gen_grad_smem(const GenericGeo& q) {
+    const size_t nx = q.n_fft > q.n_inv ? q.n_fft : q.n_inv;
+    return (2 * nx + (size_t)q.bins) * 16;
 }
 
 }  // namespace avse_gen
@@ -401,6 +498,30 @@ int avse_generic_inverse(avse_ctx* ctx, const avse_inverse_args* args, void* str
     if (bx > 1024) bx = 1024;
     if (a.out_format == AVSE_SAMPLE_I16) avse_generic_inverse_ola_kernel<short><<<dim3((unsigned)a.B, (unsigned)bx), 256, 0, st>>>(P);
     else avse_generic_inverse_ola_kernel<float><<<dim3((unsigned)a.B, (unsigned)bx), 256, 0, st>>>(P);
+    CUDA_TRY(cudaGetLastError());
+    return 0;
+}
+
+int avse_generic_inverse_backward(avse_ctx* ctx, const avse_inverse_args* args, int T_use, int t_write, const float* grad_pcm,
+                                  long long grad_pcm_stride, float* grad_mel, void* stream) {
+    const GenericGeo& q = ctx->gen.geo;
+    GenGradParams P;
+    P.a = *args;
+    P.geo = q;
+    P.d = ctx->gd;
+    P.grad = grad_pcm;
+    P.grad_stride = grad_pcm_stride;
+    P.grad_mel = grad_mel;
+    P.T_use = T_use;
+    P.t_write = t_write;
+    P.out_len = q.hop * (T_use - 1);
+    if ((long long)t_write * args->B > 0x7fffffffLL) return avse_fail(AVSE_E_ARG, "avse_inverse_backward: B * frames exceeds 2^31; split the batch");
+    const size_t smem = gen_grad_smem(q);
+    if (smem > ctx->gen_grad_smem_set) {
+        CUDA_TRY(cudaFuncSetAttribute(avse_generic_inverse_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGenMaxSmem));
+        ctx->gen_grad_smem_set = kGenMaxSmem;
+    }
+    avse_generic_inverse_grad_kernel<<<dim3((unsigned)((long long)t_write * args->B)), GEN_THREADS, smem, (cudaStream_t)stream>>>(P);
     CUDA_TRY(cudaGetLastError());
     return 0;
 }

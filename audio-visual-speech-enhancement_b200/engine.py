@@ -520,6 +520,51 @@ class SpectralEngine(object):
         check(self._lib.avse_inverse(self._ctx, ctypes.byref(a), self._stream()), "avse_inverse")
         return out
 
+    def reconstruct_differentiable(self, mixed_pcm, mel_slices, lengths=None):
+        """reconstruct (dp:60-74) as a differentiable op in the dB slices: the output is bit-identical to reconstruct's float32
+        PCM, and backward runs avse_inverse_backward, so a loss on the waveform trains the slice predictor through the fixed
+        reconstruction.  The mixture is data: a mixed_pcm that requires grad raises ValueError."""
+        mel = mel_slices if mel_slices.dim() == 4 else mel_slices.unsqueeze(0)
+        return _InverseFn.apply(mel, self, mixed_pcm, lengths, LAYOUT_SLICES)
+
+    def reconstruct_spec_differentiable(self, mixed_pcm, mel_db, lengths=None):
+        """reconstruct_spec as a differentiable op in mel_db [B, 80, T_mel] (see reconstruct_differentiable)."""
+        mel = mel_db if mel_db.dim() == 3 else mel_db.unsqueeze(0)
+        return _InverseFn.apply(mel, self, mixed_pcm, lengths, LAYOUT_SPEC)
+
+    @_on_device
+    def _inverse_launch(self, mixed_pcm, mel, lengths, layout, grad_pcm=None):
+        """avse_inverse (grad_pcm None: returns the PCM) or avse_inverse_backward (returns dL/d mel, float32, mel's shape) for a
+        contiguous float32 mel in SLICES [B, n, 80, spss] or SPEC [B, 80, T_mel] layout."""
+        B, L = mixed_pcm.shape
+        t_mel = self.spss * mel.shape[1] if layout == LAYOUT_SLICES else mel.shape[2]
+        T_use = min(t_mel, self.n_frames(L))
+        a = InverseArgs()
+        a.mel_db, a.layout = _ptr(mel), layout
+        if layout == LAYOUT_SLICES:
+            a.n_slices, a.n_frames, a.ld_t = mel.shape[1], 0, 0
+        else:
+            a.n_slices, a.n_frames, a.ld_t = 0, t_mel, t_mel
+        a.mel_stride = _rs(mel)
+        a.mixed_pcm, a.pcm_stride, a.len_pcm = _ptr(mixed_pcm), _rs(mixed_pcm), _ptr(lengths)
+        a.B, a.L = B, L
+        a.out_format = SAMPLE_F32
+        if grad_pcm is not None:
+            grad_mel = torch.empty_like(mel)
+            check(self._lib.avse_inverse_backward(self._ctx, ctypes.byref(a), _ptr(grad_pcm), _rs(grad_pcm), _ptr(grad_mel),
+                                                  self._stream()), "avse_inverse_backward")
+            return grad_mel
+        out = torch.empty((B, self.hop * (T_use - 1)), dtype=torch.float32, device=self.device)
+        per = ctypes.c_longlong(0)
+        work = None
+        if self._needs_inverse_scratch():
+            check(self._lib.avse_inverse_work_elems_ctx(self._ctx, T_use, ctypes.byref(per)), "avse_inverse_work_elems_ctx")
+            work = torch.empty((B, per.value), dtype=torch.float32, device=self.device)
+        a.out_pcm, a.out_stride = _ptr(out), _rs(out)
+        a.work, a.work_stride = _ptr(work), per.value
+        check(self._lib.avse_inverse(self._ctx, ctypes.byref(a), self._stream()), "avse_inverse")
+        return out
+
 
     # ------------------------------------------------------------------ next row f1: make_sample_set on the device
     @_on_device
@@ -573,6 +618,29 @@ class SpectralEngine(object):
         if user_perm and check and int(bad.item()):
             raise IndexError("permutation must hold %d indices in [0, %d)" % (N, N))
         return tuple(outs[:2]) + (permutation,) + tuple(outs[2:])
+
+
+class _InverseFn(torch.autograd.Function):
+    """The mixture-phase reconstruction with its vector-Jacobian product in the dB input (avse_inverse / avse_inverse_backward)."""
+
+    @staticmethod
+    def forward(ctx, mel, engine, mixed_pcm, lengths, layout):
+        if mixed_pcm.requires_grad:
+            raise ValueError("reconstruct_differentiable: mixed_pcm is data here (no gradient flows to the mixture or its phase); "
+                             "pass mixed_pcm.detach()")
+        pcm = engine._as_batch(mixed_pcm)
+        mel32 = (mel if mel.dtype == torch.float32 else mel.to(torch.float32)).contiguous()
+        ctx.engine, ctx.layout, ctx.mel_dtype = engine, layout, mel.dtype
+        ctx.save_for_backward(mel32, pcm, lengths)
+        return engine._inverse_launch(pcm, mel32, lengths, layout)
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_out):
+        mel32, pcm, lengths = ctx.saved_tensors
+        g = grad_out.to(torch.float32).contiguous()      # y.sum() hands over a stride-0 expanded tensor
+        grad_mel = ctx.engine._inverse_launch(pcm, mel32, lengths, ctx.layout, grad_pcm=g)
+        return grad_mel.to(ctx.mel_dtype), None, None, None, None
 
 
 class VideoNormalizer(object):

@@ -225,6 +225,16 @@ typedef struct avse_inverse_args {
  * on the fly) -> irfft + Hann + overlap-add / window sum-square, centre trim.  One kernel on `stream` (two for generic geometries). */
 int avse_inverse(avse_ctx* ctx, const avse_inverse_args* args, void* stream);
 
+/* Vector-Jacobian product of avse_inverse (mixture-phase form) with respect to mel_db: given grad_pcm = dL/dy
+ * [B][grad_pcm_stride] (hop * (frames_used - 1) samples per row, the forward's out_pcm shape), writes grad_mel = dL/d mel_db in
+ * mel_db's layout and mel_stride.  `args` is the avse_inverse_args of the forward call (SLICES or SPEC, len_pcm, L, B, mel_stride,
+ * ld_t) under the same validation; out_pcm and work are ignored; phase != NULL or out_format != AVSE_SAMPLE_F32 gives AVSE_E_ARG.
+ * Every frame mel_db holds is written (SPEC: columns [0, n_frames), [n_frames, ld_t) are left alone), with exact zeros for frames
+ * >= frames_used and for frames whose window sees only zero gradient.  The mixture's phase is data: no gradient flows to it.
+ * Deterministic and independent of the batch's size and order; allocates nothing; one kernel on `stream`. */
+int avse_inverse_backward(avse_ctx* ctx, const avse_inverse_args* args, const float* grad_pcm, long long grad_pcm_stride,
+                          float* grad_mel, void* stream);
+
 /* Scratch floats per utterance needed by avse_inverse for `n_frames_use` reconstructed frames (specialised geometry). */
 int avse_inverse_work_elems(int n_frames_use, long long* per_utterance);
 /* The same for the geometry of `ctx` (use this one with avse_create_ex contexts). */
