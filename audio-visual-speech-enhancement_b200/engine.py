@@ -38,6 +38,19 @@ def _on_device(fn):
     return wrapped
 
 
+def _row_array(x, B, dtype, device, name):
+    """A per-row side array (lengths: int32, SNRs: float32) as the kernels read it: a contiguous [B] tensor of `dtype` on
+    `device`.  Takes a tensor of any dtype, device or stride, a numpy array or a list; None stays None.  An int64 tensor
+    handed to the kernel as it is would be read as int32 pairs (row 1 of `[16000, 9001]` would see the high word of 16000,
+    0), so every entry point that forwards such an array converts it here.  Raises ValueError unless it holds B values."""
+    if x is None:
+        return None
+    t = x if torch.is_tensor(x) else torch.as_tensor(np.asarray(x))
+    if t.shape != (B,):
+        raise ValueError("%s: expected one value per row, shape (%d,), got %s" % (name, B, tuple(t.shape)))
+    return t.to(device=device, dtype=dtype).contiguous()
+
+
 def _rs(t):
     """Row stride in elements; a size-1 leading dimension may carry an arbitrary (even 0) stride."""
     if t is None:
@@ -181,6 +194,9 @@ class SpectralEngine(object):
         B, L = speech.shape
         assert noise.shape[0] == B and _rs(noise) == _rs(speech)
         assert noise_lengths is not None or noise.shape[1] >= L, "a noise batch narrower than the speech needs noise_lengths"
+        lengths = _row_array(lengths, B, torch.int32, self.device, "lengths")
+        noise_lengths = _row_array(noise_lengths, B, torch.int32, self.device, "noise_lengths")
+        snr_db = _row_array(snr_db, B, torch.float32, self.device, "snr_db")
         factor = torch.empty(B, dtype=torch.float32, device=self.device)
         if max_key is None:
             max_key = DbKeys(B, self.device)
@@ -210,6 +226,9 @@ class SpectralEngine(object):
         if noise is not None:
             noise = self._as_batch(noise, i16)
             assert _rs(noise) == _rs(speech) and noise.shape[0] == B
+        len_speech = _row_array(len_speech, B, torch.int32, self.device, "len_speech")
+        len_noise = _row_array(len_noise, B, torch.int32, self.device, "len_noise")
+        noise_lengths = _row_array(noise_lengths, B, torch.int32, self.device, "noise_lengths")
         T = self.n_frames(L)
         if n_slices is None:
             n_slices = self.n_slices(L)
@@ -314,6 +333,10 @@ class SpectralEngine(object):
         speech, noise = self._as_batch(speech, i16), self._as_batch(noise, i16)
         L = self.samples_per_slice * int(n_video_slices)
         n = self.n_slices(L)
+        B = speech.shape[0]        # the side arrays feed two launches: convert them once
+        lengths = _row_array(lengths, B, torch.int32, self.device, "lengths")
+        snr_db = _row_array(snr_db, B, torch.float32, self.device, "snr_db")
+        noise_lengths = _row_array(noise_lengths, B, torch.int32, self.device, "noise_lengths")
         if lengths is None and speech.shape[1] != L:
             lengths = torch.full((speech.shape[0],), speech.shape[1], dtype=torch.int32, device=self.device)
         # info: optional dict that receives the SNR factors and the dB keys
@@ -444,6 +467,7 @@ class SpectralEngine(object):
             mel = mel.unsqueeze(0)
         mel = mel.contiguous()
         B, L = mixed_pcm.shape
+        lengths = _row_array(lengths, B, torch.int32, self.device, "lengths")
         n = mel.shape[1]
         T_use = min(self.spss * n, self.n_frames(L))
         out_len = self.hop * (T_use - 1)
@@ -503,6 +527,7 @@ class SpectralEngine(object):
             mel = mel.unsqueeze(0)
         mel = mel.contiguous()
         B, L = mixed_pcm.shape
+        lengths = _row_array(lengths, B, torch.int32, self.device, "lengths")
         T_use = min(mel.shape[2], self.n_frames(L))
         out = torch.empty((B, self.hop * (T_use - 1)), dtype=torch.float32, device=self.device)
         per = ctypes.c_longlong(0)
@@ -629,6 +654,8 @@ class _InverseFn(torch.autograd.Function):
             raise ValueError("reconstruct_differentiable: mixed_pcm is data here (no gradient flows to the mixture or its phase); "
                              "pass mixed_pcm.detach()")
         pcm = engine._as_batch(mixed_pcm)
+        # one int32 copy for both launches: the backward reads the lengths the forward read
+        lengths = _row_array(lengths, pcm.shape[0], torch.int32, engine.device, "lengths")
         mel32 = (mel if mel.dtype == torch.float32 else mel.to(torch.float32)).contiguous()
         ctx.engine, ctx.layout, ctx.mel_dtype = engine, layout, mel.dtype
         ctx.save_for_backward(mel32, pcm, lengths)
