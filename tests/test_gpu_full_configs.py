@@ -90,9 +90,17 @@ def test_config5_long_form_batch_matches_oracle(eng):
         B = 64
         speech, noise = bench.synth_batch(torch, B, torch.device("cuda", 0), seed=0)
         snr = torch.tensor([bench.SNR_SWEEP[i % 5] for i in range(B)], dtype=torch.float32, device="cuda")
-        outs = eng.preprocess_pairs(speech, noise, 300, snr_db=snr)
+        info = {}
+        outs = eng.preprocess_pairs(speech, noise, 300, snr_db=snr, info=info)
         rec = eng.reconstruct(outs[3], outs[1])
         worst = _check(eng, speech, noise, outs, [0, 31, 63], 300, snr_db=snr.cpu().numpy(), inverse=rec)
+        # the statistics pass (P = 8 CTAs per utterance here): factor and equaliser within float32 rounding of numpy's float64
+        fac, eq = info["factor"].cpu().numpy(), info["keys"].equalizer.cpu().numpy()
+        for u in (0, 31, 63):
+            s, z = speech[u].double().cpu().numpy(), noise[u].double().cpu().numpy()
+            wf = np.sqrt(np.var(s) / np.var(z)) * 10.0 ** (-float(snr[u]) / 20.0)
+            wg = np.sqrt(np.sum(s * s) / np.sum(z * z))
+            assert abs(fac[u] - wf) <= 2e-7 * wf and abs(eq[u] - wg) <= 2e-7 * wg, (u, fac[u], wf, eq[u], wg)
         print("config 5 (64 x 60 s, SNR sweep): worst log-mel error %.2e dB" % worst)
     finally:
         bench.set_workload(3.0, False)

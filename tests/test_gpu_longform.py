@@ -40,9 +40,11 @@ def batch(eng):
         s, z = _pair(500 + i, n)
         S[i, :n], Z[i, :n] = s, z
     d = lambda x: torch.from_numpy(np.ascontiguousarray(x)).cuda()
-    out = eng.preprocess_pairs(d(S), d(Z), 300, lengths=d(np.array(lens, np.int32)), snr_db=d(np.array(SNRS, np.float32)))
+    info = {}
+    out = eng.preprocess_pairs(d(S), d(Z), 300, lengths=d(np.array(lens, np.int32)), snr_db=d(np.array(SNRS, np.float32)), info=info)
     torch.cuda.synchronize()
-    return S, Z, lens, out
+    # (factor, equaliser) of the statistics pass, here at P = 8 (a cluster of 8 CTAs per utterance)
+    return S, Z, lens, out, (info["factor"].cpu().numpy(), info["keys"].equalizer.cpu().numpy())
 
 
 def _oracle(S, Z, lens, i):
@@ -53,7 +55,7 @@ def _oracle(S, Z, lens, i):
 
 @pytest.mark.parametrize("i", range(5))
 def test_long_form_snr_sweep_matches_oracle(batch, i):
-    S, Z, lens, (mixed, speech, noise, pcm) = batch
+    S, Z, lens, (mixed, speech, noise, pcm), gains = batch
     r_mixed, r_speech, r_noise, r_sig = _oracle(S, Z, lens, i)
     assert tuple(mixed.shape) == (5, 300, 80, 20)
     for name, got, ref in (("mixed", mixed, r_mixed), ("speech", speech, r_speech), ("noise", noise, r_noise)):
@@ -68,10 +70,16 @@ def test_long_form_snr_sweep_matches_oracle(batch, i):
     s = S[i, :n].astype(np.float64)
     snr = 10.0 * np.log10(np.var(s) / np.var(p - s))
     assert abs(snr - SNRS[i]) < 1e-3
+    # the statistics themselves: within float32 rounding of numpy's float64 values (a partition error of one sample is ~10 ulps)
+    fac, eq = gains
+    z = Z[i, :n].astype(np.float64)
+    wf = np.sqrt(np.var(s) / np.var(z)) * 10.0 ** (-SNRS[i] / 20.0)
+    wg = np.sqrt(np.sum(s * s) / np.sum(z * z))
+    assert abs(fac[i] - wf) <= 2e-7 * wf and abs(eq[i] - wg) <= 2e-7 * wg, (i, fac[i], wf, eq[i], wg)
 
 
 def test_long_form_inverse_matches_oracle(eng, batch):
-    S, Z, lens, (mixed, speech, noise, pcm) = batch
+    S, Z, lens, (mixed, speech, noise, pcm), gains = batch
     rec = eng.reconstruct(pcm, speech)
     assert tuple(rec.shape) == (5, 160 * (6000 - 1))          # hop * (T_use - 1), Appendix B: 959 840
     for i in (0, 4):
@@ -84,7 +92,7 @@ def test_long_form_inverse_matches_oracle(eng, batch):
 
 def test_sharded_halves_equal_the_whole(eng, batch):
     # SURVEY 8(e): utterances are independent units -- processing a contiguous shard alone gives bit-identical results
-    S, Z, lens, (mixed, speech, noise, pcm) = batch
+    S, Z, lens, (mixed, speech, noise, pcm), gains = batch
     mod = importlib.import_module("audio-visual-speech-enhancement_b200.engine")
     d = lambda x: torch.from_numpy(np.ascontiguousarray(x)).cuda()
     for rank in range(2):
