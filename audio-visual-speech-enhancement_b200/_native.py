@@ -55,6 +55,7 @@ class PoolMixArgs(_c.Structure):
         ("mixed_pcm", _c.c_void_p), ("pcm_stride", _c.c_longlong),
         ("factor_out", _c.c_void_p), ("equalizer_out", _c.c_void_p),
         ("max_key", _c.c_void_p), ("min_key", _c.c_void_p), ("bad_row_flag", _c.c_void_p),
+        ("speech_start", _c.c_void_p),
     ]
 
 
@@ -64,6 +65,7 @@ EXPORTS = [
     "avse_inverse", "avse_inverse_work_elems", "avse_floor_inplace3", "avse_gather_rows",
     "avse_create_ex", "avse_get_geometry", "avse_inverse_work_elems_ctx",
     "avse_video_stats", "avse_video_normalize", "avse_mse", "avse_magphase", "avse_mix_pooled", "avse_inverse_backward",
+    "avse_gather_video",
 ]
 
 
@@ -127,6 +129,8 @@ def load(build=True):
     lib.avse_gather_rows.restype = i32
     lib.avse_mix_pooled.argtypes = [vp, _c.POINTER(PoolMixArgs), vp]
     lib.avse_mix_pooled.restype = i32
+    lib.avse_gather_video.argtypes = [vp, vp, i32, ll, i32, i32, vp, ll, vp, vp, vp, vp, vp]
+    lib.avse_gather_video.restype = i32
     _lib = lib
     return lib
 

@@ -91,6 +91,9 @@ AVSE_HD void warp_split_range(const WarpSplit& s, int block, int warp, int warps
 // Pooled pairs (avse_mix_pooled): row b of a batch mixes speech clip speech_index[b] with noise clip noise_index[b] read from
 // its sample noise_offset[b] on, n[i] = z[(off + i) mod Ln] for i < Ls -- dp:119-139 on (s, z rotated by off).  off = 0 is
 // the reference's own "double until long enough, then truncate" rule (dp:125-128).
+// With speech_start, row b is the window s = clip[a, a + Lw) of its speech clip, a = speech_start[b], Lw = min(L, Ls - a):
+// every kernel reads the row through pool_row, which hands out the window's first sample and length, so the statistics, the
+// reflect padding (mirrored inside the window) and the mix never see clip[a - 1] or clip[a + Lw].
 // ---------------------------------------------------------------------------------------------
 struct PoolRows {
     const long long* speech_index;   // [B]; nullptr: identity rows (avse_forward / avse_snr_factor batches)
@@ -100,11 +103,13 @@ struct PoolRows {
     const int* noise_len;            // [n_noise]  clip lengths (clamped to [0, noise_stride])
     long long speech_stride, noise_stride, n_speech, n_noise;
     int* bad_row_flag;               // set to 1 by the statistics pass for every invalid row (caller zeroes it)
+    const int* speech_start;         // [B] first speech sample of each row, or nullptr: the whole clip from sample 0
+    int L;                           // row length: caps the window (read only with speech_start)
 };
 
 // One resolved row: element offsets of the two clips, their lengths and the noise phase.  An invalid row (an index out of
-// range, or off outside [0, Ln) -- which includes every empty noise clip) comes back as the empty pair: both lengths 0,
-// nothing is read, factor 0, every log-mel at the amin floor.
+// range, off outside [0, Ln) -- which includes every empty noise clip --, or a speech start outside {0} u (0, Ls)) comes back
+// as the empty pair: both lengths 0, nothing is read, factor 0, every log-mel at the amin floor.
 struct PoolRow {
     long long s_off, n_off;
     int ls, ln, off;
@@ -122,8 +127,15 @@ AVSE_HD PoolRow pool_row(const PoolRows& p, int b) {
     ln = ln < 0 ? 0 : (ln < p.noise_stride ? ln : p.noise_stride);
     const int off = p.noise_offset ? p.noise_offset[b] : 0;
     r.ok = off >= 0 && off < ln;
+    long long a = 0;
+    if (p.speech_start) {                       // the window [a, a + min(L, Ls - a)); a == 0 keeps an empty clip valid
+        a = p.speech_start[b];
+        r.ok = r.ok && (a == 0 || (a > 0 && a < ls));
+        ls -= a;
+        ls = ls < p.L ? ls : p.L;
+    }
     if (!r.ok) return r;
-    r.s_off = si * p.speech_stride;
+    r.s_off = si * p.speech_stride + a;
     r.n_off = ni * p.noise_stride;
     r.ls = (int)ls; r.ln = (int)ln; r.off = off;
     return r;

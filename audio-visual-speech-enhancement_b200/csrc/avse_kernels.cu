@@ -1199,6 +1199,8 @@ extern "C" int avse_mix_pooled(avse_ctx* ctx, const avse_pool_mix_args* args, vo
     pool.n_speech = m.n_speech;
     pool.n_noise = m.n_noise;
     pool.bad_row_flag = m.bad_row_flag;
+    pool.speech_start = m.speech_start;
+    pool.L = m.L;
     avse_forward_args a = {};
     a.speech = m.speech_pool;
     a.noise = m.noise_pool;
@@ -1234,7 +1236,9 @@ extern "C" int avse_mix_pooled(avse_ctx* ctx, const avse_pool_mix_args* args, vo
     CUDA_TRY(cudaGetDevice(&dev));
     if (dev != ctx->device) return avse_fail(AVSE_E_ARG, "avse_mix_pooled: current device differs from the context's device");
 
-    const int longest = m.speech_stride < 0x7fffffffLL ? (int)m.speech_stride : 0x7fffffff;     // sizes the statistics clusters
+    // sizes the statistics clusters: a windowed row reads at most L speech samples, a whole-clip row up to the pool's stride
+    const long long reach = m.speech_start && m.L < m.speech_stride ? m.L : m.speech_stride;
+    const int longest = reach < 0x7fffffffLL ? (int)reach : 0x7fffffff;
     int rc = snr_factor_launch(ctx, m.speech_pool, m.noise_pool, m.sample_format, 0, nullptr, nullptr, m.B, longest, pool, m.snr_db,
                                m.factor_out, m.equalizer_out, m.max_key, m.min_key, stream);
     if (rc != 0) return rc;

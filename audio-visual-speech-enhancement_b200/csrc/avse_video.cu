@@ -124,6 +124,70 @@ __global__ void __launch_bounds__(256) avse_video_normalize_kernel(float* __rest
     }
 }
 
+// Video half of a training batch: dst[i] = decode(pool[index[i]]), optionally normalised like avse_video_normalize, for rows of
+// hw * frames elements (row4 float4 groups).  One CTA per output row at a time (a 128 x 128 x 5 slice is 320 KB of output), the
+// CTAs striding over the rows so any n_out fits one launch.  A thread decodes 4 consecutive elements (one uchar4 or float4 load,
+// one 16-byte store), four groups in flight; its (pixel, frame) position is walked like avse_video_normalize_kernel's.
+template <typename P> struct Pix4;
+template <> struct Pix4<unsigned char> {
+    static __device__ __forceinline__ float4 load(const unsigned char* p, long long i) {
+        const uchar4 t = __ldg(reinterpret_cast<const uchar4*>(p) + i);
+        return make_float4((float)t.x, (float)t.y, (float)t.z, (float)t.w);
+    }
+};
+template <> struct Pix4<float> {
+    static __device__ __forceinline__ float4 load(const float* p, long long i) { return __ldg(reinterpret_cast<const float4*>(p) + i); }
+};
+
+template <typename P, bool NORM>
+__global__ void __launch_bounds__(256) avse_gather_video_kernel(const P* __restrict__ pool, long long pool_slices, int row4, int frames,
+                                                                const long long* __restrict__ index, long long n_out,
+                                                                const float* __restrict__ mean, const float* __restrict__ stdv,
+                                                                float* __restrict__ dst, int* __restrict__ bad) {
+    constexpr int U = 4;                                     // float4 groups in flight per thread
+    const int step = U * blockDim.x;
+    // (pixel, frame) of the thread's first element and the advance of its position per step of 4 * blockDim.x elements
+    const int e0 = 4 * threadIdx.x;
+    const int p0 = NORM ? e0 / frames : 0, r0 = NORM ? e0 - p0 * frames : 0;
+    const int ds = NORM ? 4 * (int)blockDim.x : 0;
+    const int dp = NORM ? ds / frames : 0, dr = NORM ? ds - dp * frames : 0;
+    for (long long i = blockIdx.x; i < n_out; i += gridDim.x) {
+        const long long r = index[i];
+        if (r < 0 || r >= pool_slices) { if (threadIdx.x == 0) atomicExch(bad, 1); continue; }
+        const P* src = pool + r * (4LL * row4);
+        float4* out = reinterpret_cast<float4*>(dst) + i * row4;
+        int p = p0, q = r0;
+        for (int j0 = threadIdx.x; j0 < row4; j0 += step) {
+            float4 v[U];
+#pragma unroll
+            for (int k = 0; k < U; ++k) {
+                const int j = j0 + k * blockDim.x;
+                if (j < row4) v[k] = Pix4<P>::load(src, j);
+            }
+#pragma unroll
+            for (int k = 0; k < U; ++k) {
+                const int j = j0 + k * blockDim.x;
+                if (j >= row4) break;
+                if (NORM) {
+                    int pp = p, qq = q;
+                    auto norm = [&](float x) {                  // avse_video_normalize's arithmetic, then the next element
+                        x = (x - __ldg(mean + pp)) / __ldg(stdv + pp);
+                        if (++qq == frames) { qq = 0; ++pp; }
+                        return x;
+                    };
+                    v[k].x = norm(v[k].x);
+                    v[k].y = norm(v[k].y);
+                    v[k].z = norm(v[k].z);
+                    v[k].w = norm(v[k].w);
+                    p += dp; q += dr;
+                    if (q >= frames) { q -= frames; ++p; }
+                }
+                out[j] = v[k];
+            }
+        }
+    }
+}
+
 __global__ void __launch_bounds__(256) avse_mse_kernel(const float* __restrict__ a, const float* __restrict__ b, long long n,
                                                        double* __restrict__ acc) {
     double s = 0.0;
@@ -206,6 +270,36 @@ extern "C" int avse_video_normalize(avse_ctx* ctx, float* video, long long n_sli
     const bool vec = (total % 4) == 0 && (((size_t)video) & 15) == 0;
     if (vec) avse_video_normalize_kernel<true><<<(unsigned)bx, 256, 0, (cudaStream_t)stream>>>(video, total, hw, frames, mean, stdv);
     else avse_video_normalize_kernel<false><<<(unsigned)bx, 256, 0, (cudaStream_t)stream>>>(video, total, hw, frames, mean, stdv);
+    CUDA_TRY(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int avse_gather_video(avse_ctx* ctx, const void* pool, int pixel_format, long long pool_slices, int hw, int frames,
+                                 const long long* index, long long n_out, const float* mean, const float* stdv, float* dst,
+                                 int* bad_index_flag, void* stream) {
+    if (n_out == 0) return 0;
+    if (!ctx || !pool || !index || !dst || !bad_index_flag) return avse_fail(AVSE_E_ARG, "avse_gather_video: NULL argument");
+    if ((mean == nullptr) != (stdv == nullptr)) return avse_fail(AVSE_E_ARG, "avse_gather_video: give both mean and stdv, or neither");
+    if (pixel_format != AVSE_PIXEL_U8 && pixel_format != AVSE_PIXEL_F32) return avse_fail(AVSE_E_ARG, "avse_gather_video: bad pixel_format");
+    const long long row = (long long)hw * frames;
+    if (n_out < 0 || pool_slices <= 0 || hw <= 0 || frames <= 0 || (row & 3) || row / 4 > 0x7fffffffLL)
+        return avse_fail(AVSE_E_ARG, "avse_gather_video: bad sizes (hw * frames must be a positive multiple of 4)");
+    const size_t align = pixel_format == AVSE_PIXEL_U8 ? 3 : 15;
+    if (((size_t)pool & align) || ((size_t)dst & 15))
+        return avse_fail(AVSE_E_ARG, "avse_gather_video: dst must be 16-byte aligned, the pool aligned to 4 pixels");
+    long long bx = 8LL * ctx->num_sms;                     // 8 CTAs of 256 threads per SM, each striding over the rows
+    if (bx > n_out) bx = n_out;
+    const int row4 = (int)(row / 4);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (pixel_format == AVSE_PIXEL_U8) {
+        const unsigned char* p = static_cast<const unsigned char*>(pool);
+        if (mean) avse_gather_video_kernel<unsigned char, true><<<(unsigned)bx, 256, 0, st>>>(p, pool_slices, row4, frames, index, n_out, mean, stdv, dst, bad_index_flag);
+        else avse_gather_video_kernel<unsigned char, false><<<(unsigned)bx, 256, 0, st>>>(p, pool_slices, row4, frames, index, n_out, mean, stdv, dst, bad_index_flag);
+    } else {
+        const float* p = static_cast<const float*>(pool);
+        if (mean) avse_gather_video_kernel<float, true><<<(unsigned)bx, 256, 0, st>>>(p, pool_slices, row4, frames, index, n_out, mean, stdv, dst, bad_index_flag);
+        else avse_gather_video_kernel<float, false><<<(unsigned)bx, 256, 0, st>>>(p, pool_slices, row4, frames, index, n_out, mean, stdv, dst, bad_index_flag);
+    }
     CUDA_TRY(cudaGetLastError());
     return 0;
 }

@@ -19,6 +19,7 @@ from ._native import ForwardArgs, InverseArgs, PoolMixArgs, check
 N_FFT, HOP, N_BINS, N_MELS, SPSS = 640, 160, 321, 80, 20
 LAYOUT_SLICES, LAYOUT_SPEC = 0, 1
 SAMPLE_F32, SAMPLE_I16 = 0, 1
+PIXEL_U8, PIXEL_F32 = 0, 1
 
 
 import functools
@@ -351,7 +352,7 @@ class SpectralEngine(object):
 
     @_on_device
     def mix_pools(self, speech_pool, speech_lengths, noise_pool, noise_lengths, speech_index, noise_index, n_video_slices,
-                  noise_offset=None, snr_db=None, out=None, info=None, check=True):
+                  noise_offset=None, snr_db=None, out=None, info=None, check=True, speech_start=None):
         """preprocess_audio_pair (dp:119-139) of pairings drawn from two device-resident clip pools (avse_mix_pooled).
 
         speech_pool [Ns, >= max clip] / noise_pool [Nn, >= max clip]: float32, or int16 for both (raw WAV samples, decoded in
@@ -361,8 +362,12 @@ class SpectralEngine(object):
         (default 0 dB, dp:130).  No pairing is materialised.
         Returns (mixed, speech, noise, mixed_pcm) shaped like preprocess_pairs: [B, n, 80, spss] x3 and [B, L],
         n = int(T / spss) (dp:50, see slice_count).
-        A row with an index out of range or an offset outside [0, Ln) is invalid: it is processed as an empty pair (every slice
-        at -100 dB, PCM zeros).  check=True reads the device flag back (one synchronisation) and raises IndexError; check=False
+        speech_start [B] (optional): row b mixes the window s = clip[a : a + Lw] of its speech clip instead of the whole clip,
+        a = speech_start[b], Lw = min(L, Ls - a): the SNR statistics run over the window, the reflect padding mirrors inside it,
+        and n[i] = z[(off + i) mod Ln] for i < Lw.  Starts on slice boundaries (a = samples_per_slice * k) keep audio slice j
+        aligned with video slice k + j of the clip; any sample start is accepted.  A start is valid when a == 0 or 0 < a < Ls.
+        A row with an index out of range, an offset outside [0, Ln) or an invalid start is invalid: it is processed as an empty
+        pair (every slice at -100 dB, PCM zeros).  check=True reads the device flag back (one synchronisation) and raises IndexError; check=False
         stays asynchronous.  out: dict whose tensors are re-used from call to call (like preprocess_pairs / HostPipeline).
         info: optional dict that receives `factor` [B], the dB `keys` (DbKeys) and `valid` [B] bool = row valid and factor
         finite (a silent noise window gives inf / nan like numpy)."""
@@ -378,8 +383,10 @@ class SpectralEngine(object):
         assert ni.numel() == B and B > 0
         off = None if noise_offset is None else torch.as_tensor(noise_offset, device=dev).to(torch.int32).contiguous()
         snr = None if snr_db is None else torch.as_tensor(snr_db, device=dev).to(torch.float32).contiguous()
+        start = None if speech_start is None else torch.as_tensor(speech_start, device=dev).to(torch.int32).contiguous()
         assert off is None or off.numel() == B
         assert snr is None or snr.numel() == B
+        assert start is None or start.numel() == B
         L = self.samples_per_slice * int(n_video_slices)
         n = self.n_slices(L)
         res = {} if out is None else out
@@ -410,15 +417,20 @@ class SpectralEngine(object):
         a.mixed_pcm, a.pcm_stride = _ptr(pcm), _rs(pcm)
         a.factor_out, a.equalizer_out = _ptr(factor), _ptr(keys.equalizer)
         a.max_key, a.min_key, a.bad_row_flag = _ptr(keys.max), _ptr(keys.min), _ptr(bad)
+        a.speech_start = _ptr(start)
         _native.check(self._lib.avse_mix_pooled(self._ctx, ctypes.byref(a), self._stream()), "avse_mix_pooled")   # (`check` is the flag here)
         if info is not None:
             ok = (si >= 0) & (si < sp.shape[0]) & (ni >= 0) & (ni < nz.shape[0])
             ln = nlen[ni.clamp(0, nz.shape[0] - 1)].clamp(0, _rs(nz))
             o = torch.zeros_like(ln) if off is None else off
             ok &= (o >= 0) & (o < ln)
+            if start is not None:
+                ls = slen[si.clamp(0, sp.shape[0] - 1)].clamp(0, _rs(sp))
+                ok &= (start == 0) | ((start > 0) & (start < ls))
             info["factor"], info["keys"], info["valid"] = factor, keys, ok & torch.isfinite(factor)
         if check and int(bad.item()):
-            raise IndexError("mix_pools: a row has an index outside its pool or a noise offset outside [0, noise length)")
+            raise IndexError("mix_pools: a row has an index outside its pool, a noise offset outside [0, noise length) or a speech "
+                             "start outside [0, speech length)")
         return mixed, speech, noise, pcm
 
     @_on_device
@@ -643,6 +655,38 @@ class SpectralEngine(object):
         if user_perm and check and int(bad.item()):
             raise IndexError("permutation must hold %d indices in [0, %d)" % (N, N))
         return tuple(outs[:2]) + (permutation,) + tuple(outs[2:])
+
+    @_on_device
+    def gather_video(self, video_pool, index, normalizer=None, check=True):
+        """Video rows of a training batch (avse_gather_video): out[i] = video_pool[index[i]] decoded to float32 and, with a
+        VideoNormalizer, normalised per pixel exactly as its normalize() does (bit-identical to
+        normalizer.normalize(video_pool.float()[index])).  video_pool: uint8 or float32 device tensor whose last three dimensions
+        are one slice [H, W, F] (e.g. pack_video's [Ns, S_max, H, W, F], indexed as [Ns * S_max] slices); index: int64 slice
+        indices.  An index outside the pool leaves its row unset and, with check=True, raises IndexError (one synchronisation).
+        Returns [N, H, W, F] float32."""
+        if video_pool.dtype not in (torch.uint8, torch.float32):
+            raise ValueError("gather_video: the pool must be uint8 or float32, got %s" % video_pool.dtype)
+        if video_pool.dim() < 3 or not video_pool.is_cuda or not video_pool.is_contiguous():
+            raise ValueError("gather_video: expected a contiguous device pool [..., H, W, F]")
+        H, W, F = (int(d) for d in video_pool.shape[-3:])
+        n_pool = video_pool.numel() // max(1, H * W * F)
+        if (H * W * F) % 4:
+            raise ValueError("gather_video: H * W * F must be a multiple of 4")
+        idx = torch.as_tensor(index, device=self.device).to(torch.int64).contiguous().view(-1)
+        N = idx.numel()
+        out = torch.empty((N, H, W, F), dtype=torch.float32, device=self.device)
+        mean = stdv = None
+        if normalizer is not None:
+            assert tuple(normalizer.shape) == (H, W), "gather_video: the normaliser's image shape differs from the pool's"
+            mean, stdv = normalizer.mean_image.contiguous(), normalizer.std_image.contiguous()
+        bad = torch.zeros(1, dtype=torch.int32, device=self.device)
+        fmt = PIXEL_U8 if video_pool.dtype == torch.uint8 else PIXEL_F32
+        check_rc = self._lib.avse_gather_video(self._ctx, _ptr(video_pool), fmt, n_pool, H * W, F, _ptr(idx), N, _ptr(mean), _ptr(stdv),
+                                               _ptr(out), _ptr(bad), self._stream())
+        _native.check(check_rc, "avse_gather_video")
+        if check and N and int(bad.item()):
+            raise IndexError("gather_video: a slice index lies outside the pool's %d slices" % n_pool)
+        return out
 
 
 class _InverseFn(torch.autograd.Function):
@@ -906,6 +950,31 @@ def pack_clips(clips, device=None, dtype=torch.float32, allow_empty=True):
     return torch.from_numpy(host).to(device), torch.from_numpy(lengths.astype(np.int32)).to(device)
 
 
+def pack_video(clips, device=None, dtype=torch.uint8):
+    """A list of per-clip video slices [S_k, H, W, F] (numpy arrays or tensors) -> (pool [N, S_max, H, W, F], counts [N] int32)
+    on `device`: clip k's slices in row k, zeros after its count.  dtype torch.uint8 keeps the decoder's pixels (a quarter of
+    the float32 bytes; values must be integers in [0, 255]), torch.float32 stores them as they are.  SpectralEngine.gather_video
+    and DynamicMixer.sample_set decode and normalise the slices they gather."""
+    if dtype not in (torch.uint8, torch.float32):
+        raise ValueError("pack_video: dtype must be torch.uint8 or torch.float32")
+    datas = [c.detach().cpu().numpy() if torch.is_tensor(c) else np.asarray(c) for c in clips]
+    if not datas:
+        raise ValueError("pack_video: no clips")
+    shape = None
+    for k, d in enumerate(datas):
+        if d.ndim != 4 or (shape is not None and d.shape[1:] != shape):
+            raise ValueError("pack_video: clip %d has shape %s; expected [slices, H, W, F] like the others" % (k, d.shape))
+        shape = d.shape[1:]
+        if dtype == torch.uint8 and d.dtype != np.uint8 and d.size:
+            if not (np.all(d >= 0) and np.all(d <= 255) and np.all(d == np.round(d))):
+                raise ValueError("pack_video: clip %d holds values that are not uint8 pixels; pack it as float32" % k)
+    counts = np.array([d.shape[0] for d in datas], dtype=np.int64)
+    host = np.zeros((len(datas), max(1, int(counts.max()))) + tuple(shape), dtype=np.uint8 if dtype == torch.uint8 else np.float32)
+    for k, d in enumerate(datas):
+        host[k, :d.shape[0]] = d
+    return torch.from_numpy(host).to(device), torch.from_numpy(counts.astype(np.int32)).to(device)
+
+
 def draw_pairings(generator, B, n_speech, noise_lengths, snr_db=(-10.0, 10.0)):
     """The random pairing of one DynamicMixer epoch, drawn on the host from `generator` (a CPU torch.Generator: the same seed
     gives the same pairing on any machine).  Returns CPU tensors (speech_index int64, noise_index int64, noise_offset int32,
@@ -943,24 +1012,32 @@ class DynamicMixer(object):
     without materialising any pairing (SpectralEngine.mix_pools).  The reference mixes each speech file with one noise file
     once, at 0 dB from noise sample 0, and re-reads those frozen mixtures every epoch (speech_enhancer.py:17-58).
 
-    All clips of a mixer share one n_video_slices (L = samples_per_slice * n_video_slices): a corpus with several
-    durations builds one mixer per duration, as preprocess_data buckets.  Pairings come from the mixer's own torch.Generator
-    (seeded with `seed`): the same seed and the same sequence of calls give bit-identical epochs.  In a multi-GPU job give
-    every rank its own seed.
+    Every row is L = samples_per_slice * n_video_slices samples long.  Without clip_slices a row is the start of its speech
+    clip (all clips of such a mixer should share one duration, as preprocess_data buckets).  With clip_slices [Ns] -- each
+    speech clip's min(video, audio) slice count (dp:164) -- clips of any length share one mixer: every row is a window that
+    starts on a random slice boundary k of its clip, k uniform in [0, max(0, clip_slices[s] - n_video_slices)], so every part
+    of a long clip is trained on.  video_pool = pack_video(...)'s (pool, counts) lets sample_set gather the matching video
+    slices on the device.
 
-    One epoch, chained into make_sample_set (video rows are indexed by speech_index, like the reference's sample list)::
+    Pairings come from the mixer's own torch.Generator (seeded with `seed`), window starts from a second one seeded from the
+    same `seed`: the same seed and the same sequence of calls give bit-identical epochs, and the pairings of a seed are the
+    same with and without windows.  In a multi-GPU job give every rank its own seed.
+
+    One epoch::
 
         speech_pool, speech_len = pack_clips(speech_clips, eng.device)
         noise_pool, noise_len = pack_clips(noise_clips, eng.device, allow_empty=False)
-        mixer = DynamicMixer(eng, speech_pool, speech_len, noise_pool, noise_len, n_video_slices=15, snr_db=(-10.0, 10.0), seed=rank)
+        video = pack_video(video_clips, eng.device)                     # uint8 [Ns, S_max, H, W, F], counts [Ns]
+        mixer = DynamicMixer(eng, speech_pool, speech_len, noise_pool, noise_len, n_video_slices=15, snr_db=(-10.0, 10.0),
+                             seed=rank, clip_slices=clip_slices, video_pool=video)
         for epoch in range(n_epochs):
-            pairing = mixer.draw(3 * len(speech_clips))            # three noisy versions of every clip per epoch
+            pairing = mixer.draw(3 * len(speech_clips))                 # three noisy windows of every clip per epoch
             mixed, speech, noise, pcm, valid = mixer.mix(pairing)
-            n = torch.where(valid, clip_slices[pairing[0]], 0)     # clip_slices: min(video, audio) slices per speech clip
-            X_mixed, X_speech, perm = eng.make_sample_set(mixed, speech, n_slices=n)
+            X_video, X_mixed, X_speech, perm = mixer.sample_set(pairing, mixed, speech, valid, normalizer=normalizer)
     """
 
-    def __init__(self, engine, speech_pool, speech_lengths, noise_pool, noise_lengths, n_video_slices, snr_db=(-10.0, 10.0), seed=0):
+    def __init__(self, engine, speech_pool, speech_lengths, noise_pool, noise_lengths, n_video_slices, snr_db=(-10.0, 10.0), seed=0,
+                 clip_slices=None, video_pool=None):
         self.eng = engine
         self.device = engine.device
         self.speech_pool, self.noise_pool = speech_pool, noise_pool
@@ -973,20 +1050,92 @@ class DynamicMixer(object):
         self.snr_db = snr_db
         self.generator = torch.Generator()
         self.generator.manual_seed(int(seed))
+        Ns = speech_pool.shape[0]
+        self.clip_slices = None
+        if clip_slices is not None:
+            cs = torch.as_tensor(np.asarray(clip_slices) if not torch.is_tensor(clip_slices) else clip_slices).to("cpu", torch.int64)
+            if cs.shape != (Ns,) or bool((cs < 0).any()):
+                raise ValueError("DynamicMixer: clip_slices must hold one slice count >= 0 per speech clip (%d)" % Ns)
+            self._clip_slices_host = cs
+            self.clip_slices = cs.to(self.device)
+            # window starts: a second generator, so the pairing sequence of a seed does not depend on whether windows are drawn
+            self.start_generator = torch.Generator()
+            self.start_generator.manual_seed((int(seed) * 0x9E3779B97F4A7C15 + 0x632BE59BD9B4E019) % (1 << 64))
+        self.video_pool = self.video_counts = None
+        if video_pool is not None:
+            pool, counts = video_pool
+            counts = torch.as_tensor(counts).to("cpu", torch.int64)
+            if self.clip_slices is None:
+                raise ValueError("DynamicMixer: video_pool needs clip_slices (the slices of each clip the audio may use)")
+            if pool.dim() != 5 or pool.shape[0] != Ns or counts.shape != (Ns,):
+                raise ValueError("DynamicMixer: video_pool must be pack_video's (pool [Ns, S_max, H, W, F], counts [Ns])")
+            if bool((self._clip_slices_host > counts).any()):
+                raise ValueError("DynamicMixer: clip_slices exceeds the video slices stored for a clip")
+            self.video_pool = pool.to(self.device).contiguous()
+            self.video_counts = counts.to(self.device)
 
     def draw(self, B):
-        """(speech_index, noise_index, noise_offset, snr_db) device tensors of B fresh rows (see draw_pairings)."""
+        """(speech_index, noise_index, noise_offset, snr_db) device tensors of B fresh rows (see draw_pairings); with
+        clip_slices, a fifth tensor speech_start [B] int32 = samples_per_slice * k, k uniform in
+        [0, max(0, clip_slices[speech_index] - n_video_slices)]."""
         pairing = draw_pairings(self.generator, B, self.speech_pool.shape[0], self._noise_lengths_host, self.snr_db)
+        if self.clip_slices is not None:
+            kmax = (self._clip_slices_host[pairing[0]] - self.n_video_slices).clamp(min=0)
+            u = torch.rand(int(B), generator=self.start_generator, dtype=torch.float64)
+            k = torch.minimum((u * (kmax + 1).to(torch.float64)).to(torch.int64), kmax)
+            pairing = pairing + ((k * self.eng.samples_per_slice).to(torch.int32),)
         return tuple(t.to(self.device) for t in pairing)
 
     def mix(self, pairing, out=None):
-        """mix_pools of a drawn pairing: (mixed, speech, noise, mixed_pcm, valid), valid [B] bool = factor finite (a silent noise
-        window gives inf / nan).  Asynchronous: nothing is read back."""
+        """mix_pools of a drawn pairing (4-tuple, or 5-tuple with speech_start): (mixed, speech, noise, mixed_pcm, valid),
+        valid [B] bool = row valid and factor finite (a silent noise window gives inf / nan).  Asynchronous: nothing is read
+        back."""
         info = {}
-        si, ni, off, snr = pairing
+        si, ni, off, snr = pairing[:4]
+        start = pairing[4] if len(pairing) > 4 else None
         mixed, speech, noise, pcm = self.eng.mix_pools(self.speech_pool, self.speech_lengths, self.noise_pool, self.noise_lengths, si, ni,
-                                                       self.n_video_slices, noise_offset=off, snr_db=snr, out=out, info=info, check=False)
+                                                       self.n_video_slices, noise_offset=off, snr_db=snr, out=out, info=info, check=False,
+                                                       speech_start=start)
         return mixed, speech, noise, pcm, info["valid"]
+
+    def _rows(self, pairing, n, valid):
+        """Per row: its first video slice k_b (speech_start / samples_per_slice) and kept slice count n_b."""
+        si = pairing[0].to(self.device, torch.int64)
+        k = torch.zeros_like(si)
+        if len(pairing) > 4:
+            k = pairing[4].to(self.device, torch.int64) // self.eng.samples_per_slice
+        if self.clip_slices is not None:
+            nb = (self.clip_slices[si] - k).clamp(0, n)
+        else:
+            nb = torch.full_like(si, n)
+        nb = torch.where(torch.as_tensor(valid, device=self.device), nb, torch.zeros_like(nb))
+        return si, k, nb
+
+    def sample_set(self, pairing, mixed, speech, valid, normalizer=None, permutation=None, generator=None):
+        """make_sample_set of one mixed batch together with its video: (video [N, H, W, F] float32, X_mixed, X_speech,
+        permutation).  Row b keeps n_b = min(clip_slices[s_b] - k_b, n) slices (n = the batch's slice count, k_b = the window's
+        first slice, 0 without windows; 0 slices for a row that is not valid).  Video row r is slice k_b + j of clip s_b where
+        (b, j) is concatenated row permutation[r], so video and audio rows stay paired; with a VideoNormalizer it is normalised
+        as normalizer.normalize would.  video is None when the mixer has no video_pool."""
+        n = int(mixed.shape[1])
+        si, k, nb = self._rows(pairing, n, valid)
+        X_mixed, X_speech, perm = self.eng.make_sample_set(mixed, speech, n_slices=nb, permutation=permutation, generator=generator)
+        video = None
+        if self.video_pool is not None:
+            index = video_slice_index(si, k, nb, n, int(self.video_pool.shape[1]), perm)
+            video = self.eng.gather_video(self.video_pool, index, normalizer=normalizer, check=False)
+        return video, X_mixed, X_speech, perm
+
+
+def video_slice_index(speech_index, first_slice, n_slices, n, s_max, permutation):
+    """Video slice indices (into a pack_video pool flattened to [Ns * s_max] slices) of the concatenated rows permutation[r],
+    in make_sample_set's order (sample-major, slice-minor, rows j < n_slices[b] of each sample b of n): concatenated row (b, j)
+    is clip speech_index[b], slice first_slice[b] + j.  All tensors on one device; returns int64 [N]."""
+    dev = speech_index.device
+    j = torch.arange(int(n), device=dev, dtype=torch.int64)
+    keep = j.unsqueeze(0) < n_slices.to(dev, torch.int64).unsqueeze(1)
+    src = (speech_index.to(torch.int64) * int(s_max) + first_slice.to(dev, torch.int64)).unsqueeze(1) + j.unsqueeze(0)
+    return src[keep][torch.as_tensor(permutation, device=dev, dtype=torch.int64)].contiguous()
 
 
 def fit_noise(noise, n_noise, n_speech_max):

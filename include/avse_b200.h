@@ -147,10 +147,17 @@ int avse_floor_inplace3(avse_ctx* ctx, float* speech, float* noise, float* mixed
  * clip with the noise n[i] = z[(off + i) mod Ln], i < Ls, where z = the first Ln = noise_len[noise_index[b]] samples of that
  * noise clip and off = noise_offset[b]: off = 0 is the reference's own rule (tile a short noise, dp:125-126, truncate a long
  * one, dp:128).  factor = sqrt(var(s) / var(n)) * 10^(-snr_db[b]/20) over the Ls samples (dp:130, float64 sums); the speech
- * always starts at its sample 0 (its video slices are aligned to it, dp:164) and is zero padded / truncated to L (dp:36-42).
+ * starts at its sample 0 (its video slices are aligned to it, dp:164) unless speech_start gives a window (below), and is zero
+ * padded / truncated to L (dp:36-42).
  * A row is INVALID when an index is out of range or off is outside [0, Ln) (so every empty noise clip): it reads no sample,
  * is processed as an empty pair (factor 0, every slice at the amin floor -100 dB, PCM zeros) and sets *bad_row_flag.
  * A silent noise window gives inf / nan like numpy (avse_snr_factor).
+ * Windows: with speech_start != NULL, row b is the same computation on the window s = clip[a, a + Lw) of its speech clip,
+ * a = speech_start[b], Lw = min(L, Ls - a): the statistics run over the Lw window samples, the noise is n[i] = z[(off + i)
+ * mod Ln] for i < Lw, librosa's reflect padding mirrors inside the window (clip[a - 1] and clip[a + Lw] are never read) and
+ * the PCM is zero padded to L.  A start is valid when a == 0 or 0 < a < Ls; any other start makes the row invalid.  Any
+ * sample start is accepted; a start on a slice boundary (a = k * samples_per_slice) keeps audio slice j aligned with video
+ * slice k + j of the clip.
  * Enqueues the statistics pass, the forward pass and avse_floor_inplace3 on `stream`; allocates nothing.  Works on every
  * context avse_forward serves pair batches on (F4, 2-frame and generic-geometry kernels), float32 or int16 pools under the
  * same rules as avse_forward. */
@@ -185,6 +192,8 @@ typedef struct avse_pool_mix_args {
     int* max_key;                   /* [B][3] caller scratch (running dB maxima), required */
     int* min_key;                   /* [B][3] caller scratch (running minima: lets the floor skip rows), or NULL */
     int* bad_row_flag;              /* device int the caller zeroed; set to 1 when any row is invalid; required */
+    /* speech windows (appended: a zero-initialised struct keeps the whole-clip rows above) */
+    const int* speech_start;        /* [B] int32 first speech sample of each row, or NULL: every row from sample 0 */
 } avse_pool_mix_args;
 
 int avse_mix_pooled(avse_ctx* ctx, const avse_pool_mix_args* args, void* stream);
@@ -255,6 +264,18 @@ int avse_max_db(avse_ctx* ctx, const int* max_key, int n, float* out_db, void* s
 int avse_gather_rows(avse_ctx* ctx, const float* src0, const float* src1, const float* src2, long long src_rows,
                      long long row_elems, const long long* index, long long n_out, float* dst0, float* dst1, float* dst2,
                      int* bad_index_flag, void* stream);
+
+/* Video half of a training batch (the video rows of make_sample_set): dst[i][e] = decode(pool[index[i]][e]) for e < hw * frames,
+ * normalised as avse_video_normalize does when mean / stdv ([hw] float32) are given: (x - mean[p]) / stdv[p], p = e / frames,
+ * the same IEEE division.  pool: [pool_slices][hw][frames] of AVSE_PIXEL_U8 (decoder pixels, 4-byte aligned) or AVSE_PIXEL_F32
+ * (16-byte aligned) elements; dst: float32 [n_out][hw * frames], 16-byte aligned; hw * frames a multiple of 4.  index: int64
+ * [n_out] on the device, values in [0, pool_slices); an out-of-range value sets *bad_index_flag (device int the caller zeroed)
+ * and leaves that output row untouched.  Any n_out >= 0 (0: nothing is enqueued).  Allocates nothing. */
+#define AVSE_PIXEL_U8 0  /* uint8 pixels */
+#define AVSE_PIXEL_F32 1 /* float32 pixels */
+int avse_gather_video(avse_ctx* ctx, const void* pool, int pixel_format, long long pool_slices, int hw, int frames,
+                      const long long* index, long long n_out, const float* mean, const float* stdv, float* dst,
+                      int* bad_index_flag, void* stream);
 
 /* VideoNormalizer.__init__ (dp:201-205): per-pixel mean and population std over (slices, frames) of the mouth-crop tensor
  * video [n_slices][hw][frames] float32 (hw = height * width, e.g. 128 * 128; frames = 5).  scratch: 2 * hw doubles
